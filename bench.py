@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- particle-steps/sec of the filtering recursion on B200 (contract: task statement section 4).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c1|c2] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c1|c2] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is ONE pass of the hot path over one batch of synthetic trajectories: the whole
 ``forward_loop`` of the named BASELINE config (T filter steps for N trajectories).
@@ -19,6 +19,11 @@ A "step" is ONE pass of the hot path over one batch of synthetic trajectories: t
                 this box" -- launch-bound, ~150-200 library kernels per filter step).
   training      BASELINE config C4 at the same rank count: one BPTT step (forward over 15 filter steps, backward,
                 gradient all-reduce over NCCL, Adam) captured in ONE CUDA graph per rank; ms/step max over ranks.
+
+--dump-outputs DIR (c1, c2, c3): after the timed steps of ``value``, rank 0 writes what the last of them computed as
+DIR/<name>.npy (float32): the estimates of every filter step, and the belief the filter holds afterwards (particle
+states and log-weights; for the EKF, the fused covariances).  The device noise is seeded, so with the same arguments the
+inputs are identical from run to run and two builds can be compared output for output.
 
 Multi-GPU: trajectories are sharded, N per rank is fixed (weak scaling), no data-path collective.
 """
@@ -53,6 +58,7 @@ WORKLOADS = {
 CPU_SAMPLE = {"c3": (64, 20), "c4": (256, 15)}
 GPU_EAGER_SAMPLE = {"c3": (512, 20), "c1": (32, 50), "c2": (256, 100)}  # eager-torch oracle on the GPU (launch-bound)
 FLOP_PER_PARTICLE_STEP = {2: 189_824.0, 3: 190_336.0}  # BASELINE.md section 4 (hoisted minimum)
+DUMP_LIMIT_BYTES = 64_000_000  # C3's estimates + final particle set: 52.4 MB
 
 
 def measured_peaks():
@@ -131,6 +137,18 @@ def build_inputs(workload, seed=0):
     name, sd, N, M, T, _ = WORKLOADS[workload]
     states, obs, controls = synthetic_trajectories(T + 1, N, sd, seed=seed)
     return states, obs, controls
+
+
+def dump_outputs(directory, outputs):
+    """Write every tensor of ``outputs`` (name -> tensor) as ``directory/<name>.npy`` in float32."""
+    import numpy as np
+
+    arrays = {name: t.detach().float().cpu().numpy() for name, t in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, f"outputs of {total} bytes exceed the dump limit of {DUMP_LIMIT_BYTES}"
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 def run_cpu_oracle(workload, n_sample, t_sample, repeats=1, warm=True, device="cpu"):
@@ -515,7 +533,13 @@ def main():
     ap.add_argument("--precision", default=None, choices=["fp32", "bf16x3", "bf16"])
     ap.add_argument("--resample-mode", default="multinomial")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (workloads c1, c2, c3)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload in ("c4", "c5")):
+        ap.error("--dump-outputs covers the forward workloads c1, c2 and c3 of --impl b200")
     if os.environ.get("MMF_BENCH_WATCHDOG_S"):  # diagnosis of a hung rank: dump every thread's stack and exit
         import faulthandler
         faulthandler.dump_traceback_later(float(os.environ["MMF_BENCH_WATCHDOG_S"]), exit=True)
@@ -590,7 +614,7 @@ def main():
             with torch.no_grad():
                 filt.initialize_beliefs(mean=dev_mean0, covariance=cov)
                 means, covs = filt._advance(filters, dev_controls, z, r)
-                return ops.kf_fuse_crossmodal(means, covs, beta)[0]
+                return ops.kf_fuse_crossmodal(means, covs, beta)  # fused means, fused covariances
 
     def e2e_pass():
         with torch.no_grad():
@@ -615,10 +639,11 @@ def main():
         barrier()
         ops.PROFILE.reset(enabled=profile)
         start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        out = None
         with ClockSampler(local_rank) as clk:
             start.record()
             for _ in range(steps):
-                fn()
+                out = fn()
             stop.record()
             barrier()
         ms = start.elapsed_time(stop)
@@ -627,22 +652,29 @@ def main():
         t = torch.tensor([ms], device=dev, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return t.item() / steps, clk.summary(), prof
+        return t.item() / steps, clk.summary(), prof, out
 
     # inputs per pass (>= 100 MB of particle state + features) exceed nothing like L2 reuse across passes:
     # every step rewrites the N*M particle set (C3: 49 MB states+weights per step, new noise each step).
-    ms_resident, clocks, prof = timed(resident_pass, args.steps, args.warmup, profile=True)
+    torch.manual_seed(rank)  # the device noise of every pass: the same draws from run to run
+    ms_resident, clocks, prof, last = timed(resident_pass, args.steps, args.warmup, profile=True)
+    if args.dump_outputs and rank == 0:
+        if is_pf:
+            dump_outputs(args.dump_outputs, {"estimates": last, "particle_states": filt.particle_states,
+                                             "particle_log_weights": filt.particle_log_weights})
+        else:
+            dump_outputs(args.dump_outputs, {"estimates": last[0], "covariances": last[1]})
     # kernel-level numbers: the same kernels launched step by step (one C call per kernel, CUDA events around each on the
     # launching stream) instead of through the whole-sequence call, which offers no place to put an event
     ms_profiled = None
     if is_pf:
         filt.whole_loop = False
         saved_graph, filt.graph_max_particles = filt.graph_max_particles, 0
-        ms_profiled, _, prof_k = timed(resident_pass, max(1, min(args.steps, 2)), 1, profile=True)
+        ms_profiled, _, prof_k, _ = timed(resident_pass, args.steps, 1, profile=True)
         filt.whole_loop, filt.graph_max_particles = True, saved_graph
         prof["kernels"].update(prof_k["kernels"])
     # same step / warm-up counts as `value` (small workloads capture their CUDA graph on the second call: warm-up)
-    ms_e2e, clocks_e2e, _ = timed(e2e_pass, args.steps, args.warmup)
+    ms_e2e, clocks_e2e, _, _ = timed(e2e_pass, args.steps, args.warmup)
 
     # ---- the HBM-bound kernel of the step, stand-alone, per resampling mode (north star: >= 60 % of the HBM roofline) ----
     hbm_modes = None
@@ -679,7 +711,7 @@ def main():
         filt.particle_states = filt.particle_log_weights = None
         torch.cuda.empty_cache()
         try:
-            tr = run_c4(ctx, max(args.steps, 5), args.warmup, args.precision)
+            tr = run_c4(ctx, args.steps, args.warmup, args.precision)
             line["training"] = {k: tr[k] for k in ("value", "unit", "n_gpus", "ms_per_step", "steps", "dtype", "config", "clocks")}
             line["training"]["kernels"] = tr["kernels"]
         except Exception as exc:  # the forward line above is measured: a failing training record must not take it down
@@ -700,8 +732,8 @@ def main():
                 "share_of_step": k["avg_ms"] * T / ms_resident,
                 "timed_in": "a pass that launches the kernels step by step (CUDA events per launch); value / ms_per_step "
                             "come from the whole-sequence call (mmf_pf_forward_loop)", "ms_per_step_profiled_pass": ms_profiled,
-                "other_kernels": {n: {"avg_ms": v["avg_ms"], "count_per_pass": v["count"] / max(1, min(args.steps, 2)),
-                                      "share": v["avg_ms"] * v["count"] / max(1, min(args.steps, 2)) / ms_resident}
+                "other_kernels": {n: {"avg_ms": v["avg_ms"], "count_per_pass": v["count"] / args.steps,
+                                      "share": v["avg_ms"] * v["count"] / args.steps / ms_resident}
                                   for n, v in prof["kernels"].items() if n not in ("pf_predict_measure", "pf_forward_loop")},
             }
             nr = prof["kernels"].get("pf_normalize_resample")

@@ -14,6 +14,7 @@ import multimodalfilter_b200 as mmf
 from multimodalfilter_b200 import _lib, fused
 from multimodalfilter_b200.crossmodal import models as M
 from multimodalfilter_b200.synthetic import fill_parameters, synthetic_trajectories
+from oracle.make_golden import REFERENCE, reference_available
 
 from util import REPO, header_symbols, run_packed_chain, run_packed_rows
 
@@ -173,9 +174,9 @@ def test_install_aliases_make_reference_imports_resolve():
         "from fannypack.nn import resblocks\n"
         "import torchfilter.types as types\n"
         "assert torchfilter.filters.ParticleFilter.__module__.startswith('multimodalfilter_b200')\n"
-        "import os\n"
-        "if os.path.isdir('/root/reference/crossmodal'):\n"
-        "    sys.path.insert(1, '/root/reference')\n"
+        "reference = %r\n"
+        "if reference:\n"
+        "    sys.path.insert(1, reference)\n"
         "    import warnings; warnings.filterwarnings('ignore')\n"
         "    import crossmodal\n"
         "    from multimodalfilter_b200 import fused\n"
@@ -184,7 +185,7 @@ def test_install_aliases_make_reference_imports_resolve():
         "    k = crossmodal.door_models.DoorCrossmodalKalmanFilter()\n"
         "    assert fused.EKFPlan.build(list(k.filter_models)) is not None\n"
         "print('OK')\n"
-    ) % REPO
+    ) % (REPO, REFERENCE if reference_available() else None)
     res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
     assert res.returncode == 0 and "OK" in res.stdout, res.stderr[-3000:]
 

@@ -37,14 +37,16 @@ def test_fixture_is_finite_and_nontrivial(golden):
 
 
 def test_reference_still_agrees_when_mounted(golden):
-    """Where /root/reference exists (the build container) re-run the reference itself in a
-    subprocess and compare with the committed fixture; skipped on the GPU box."""
+    """Where MMF_REFERENCE_DIR names a checkout of the reference, re-run the reference itself in a
+    subprocess and compare with the committed fixture; skipped without one."""
     import os
     import subprocess
     import sys
 
-    if not os.path.isdir("/root/reference/crossmodal"):
-        pytest.skip("reference not mounted")
+    from oracle.make_golden import reference_available
+
+    if not reference_available():
+        pytest.skip("MMF_REFERENCE_DIR does not name a checkout of the reference")
     repo = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     code = (
         "import sys; sys.path.insert(0, %r)\n"

@@ -1,8 +1,8 @@
 """Training-loop glue (SURVEY.md section 8f rank 3): ``torchfilter.data`` / ``torchfilter.train`` / ``fannypack.utils.Buddy``
-drop-ins.  CPU part: the reference's OWN ``crossmodal/train_helpers.py`` (imported from /root/reference when it is there)
-runs unchanged on top of ``multimodalfilter_b200.install()`` for the phases that are plain torch modules.  GPU part:
-``train_e2e`` (ref: crossmodal/train_helpers.py:124-162), restated call for call because /root/reference does not travel
-to the GPU box, trains a PushCrossmodalParticleFilter through the fused BPTT kernels."""
+drop-ins.  CPU part: the reference's OWN ``crossmodal/train_helpers.py`` (imported from the checkout of the reference that
+MMF_REFERENCE_DIR names, when there is one) runs unchanged on top of ``multimodalfilter_b200.install()`` for the phases
+that are plain torch modules.  GPU part: ``train_e2e`` (ref: crossmodal/train_helpers.py:124-162), restated call for call
+so that it runs without the reference, trains a PushCrossmodalParticleFilter through the fused BPTT kernels."""
 import os
 import subprocess
 import sys
@@ -10,6 +10,8 @@ import sys
 import numpy as np
 import pytest
 import torch
+
+from oracle.make_golden import REFERENCE, reference_available
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -74,7 +76,7 @@ def test_buddy_minimize_and_checkpoint(tmp_path):
     assert model[2].weight.abs().sum() > 0
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/crossmodal"), reason="the reference tree is not mounted")
+@pytest.mark.skipif(not reference_available(), reason="MMF_REFERENCE_DIR does not name a checkout of the reference")
 def test_reference_train_helpers_run_on_the_drop_in():
     """ref: crossmodal/train_helpers.py, imported unchanged: configure() + the three pre-training phases whose models are
     plain torch modules (dynamics single-step / recurrent, PF measurement, virtual sensor) on CPU."""
@@ -84,7 +86,7 @@ sys.path.insert(0, %r); sys.path.insert(1, %r)
 warnings.filterwarnings("ignore")
 import multimodalfilter_b200 as mmf; mmf.install()
 import fannypack, torch, torchfilter
-sys.path.insert(2, "/root/reference")
+sys.path.insert(2, %r)
 import crossmodal
 from crossmodal import train_helpers
 from test_training_glue import _trajectories
@@ -104,7 +106,7 @@ train_helpers.configure(buddy=buddy2, trajectories=_trajectories(3, 6, 3), num_w
 train_helpers.train_virtual_sensor(epochs=1, batch_size=5)
 assert buddy2.optimizer_steps == 3
 print("OK")
-''' % (REPO, os.path.join(REPO, "tests"))
+''' % (REPO, os.path.join(REPO, "tests"), REFERENCE)
     res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=900)
     assert res.returncode == 0 and "OK" in res.stdout, (res.stdout[-2000:], res.stderr[-3000:])
 
