@@ -138,9 +138,8 @@ __global__ void __launch_bounds__(RF_TPB, NG <= 4 ? 7 : 4) k_resample_fast(const
       dst[1] = make_float4(e[g][4], e[g][5], e[g][6], e[g][7]);
     }
     __syncwarp();
-    // ---- estimate: sum_j e_j x_j (divided by the total below) or arg max ---------------------------------------
+    // ---- estimate: sum_j e_j x_j (divided by the total below); the arg max waits for the total --------------------
     float acc[MMF_MAX_SD] = {0.f, 0.f, 0.f, 0.f};
-    int best_i = 0x7fffffff;
     if (P.logits_in == nullptr) {
       const float* xs = P.states + (size_t)n * M * sd;
       if (P.estimation == MMF_ESTIMATE_WEIGHTED_AVERAGE) {
@@ -163,18 +162,6 @@ __global__ void __launch_bounds__(RF_TPB, NG <= 4 ? 7 : 4) k_resample_fast(const
         }
 #pragma unroll
         for (int d = 0; d < MMF_MAX_SD; ++d) acc[d] = warp_sum(acc[d]);
-      } else {
-        // first particle whose weight equals the maximum (e is monotone in the log-weight; e == 1 exactly at the max)
-        float best = -1.0f;
-        for (int j = lane; j < M; j += 32) {
-          const float w = cdf[j];
-          if (w > best) { best = w; best_i = j; }
-        }
-        const float gbest = warp_max(best);
-        int cand = best == gbest ? best_i : 0x7fffffff;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) cand = min(cand, __shfl_xor_sync(0xffffffffu, cand, o));
-        best_i = cand == 0x7fffffff ? 0 : cand;
       }
     }
     // ---- CDF in registers: the blocked order of the FAST definition ------------------------------------------------
@@ -210,6 +197,7 @@ __global__ void __launch_bounds__(RF_TPB, NG <= 4 ? 7 : 4) k_resample_fast(const
     __syncwarp();
     const float total = cdf[M - 1];
     const float scale = (float)K / total;
+    const float lse = mx + logf(total);
     // ---- per-trajectory outputs ------------------------------------------------------------------------------------
     if (P.logits_in == nullptr) {
       if (P.estimation == MMF_ESTIMATE_WEIGHTED_AVERAGE) {
@@ -220,16 +208,29 @@ __global__ void __launch_bounds__(RF_TPB, NG <= 4 ? 7 : 4) k_resample_fast(const
             if (lane == d) v = acc[d];
           P.est_out[(size_t)n * sd + lane] = __fdiv_rn(v, total);
         }
-      } else if (lane < sd) {
-        P.est_out[(size_t)n * sd + lane] = P.states[((size_t)n * M + best_i) * sd + lane];
+      } else {
+        // first arg max of the normalised log-weights fl(l_j - lse), as every other path takes it.  Not of e_j: two
+        // log-weights less than half an ulp of lse apart normalise to the same value (the first one wins), while their
+        // exponentials on the un-normalised scale still differ.
+        float best = -INFINITY;
+        int best_i = 0x7fffffff;
+        for (int j = lane; j < M; j += 32) {
+          const float l = __fsub_rn(__ldg(lw + j), lse);
+          if (l > best) { best = l; best_i = j; }
+        }
+        const float gbest = warp_max(best);
+        int cand = best == gbest ? best_i : 0x7fffffff;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) cand = min(cand, __shfl_xor_sync(0xffffffffu, cand, o));
+        best_i = cand == 0x7fffffff ? 0 : cand;
+        if (lane < sd) P.est_out[(size_t)n * sd + lane] = P.states[((size_t)n * M + best_i) * sd + lane];
       }
     }
     if (P.logits_out || P.logw_norm_out) {  // debug / introspection only
-      const float lse = mx + logf(total);
       for (int j = lane; j < M; j += 32) {
         const float l = lw[j];
         if (P.logits_out) P.logits_out[(size_t)n * M + j] = l;
-        if (P.logw_norm_out) P.logw_norm_out[(size_t)n * M + j] = l - lse;
+        if (P.logw_norm_out) P.logw_norm_out[(size_t)n * M + j] = __fsub_rn(l, lse);
       }
     }
     // ---- guide table: guide[b] = number of CDF entries whose bucket is < b = first entry whose bucket is >= b ----------
