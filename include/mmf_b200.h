@@ -218,6 +218,31 @@ int mmf_ekf_loop_fwd(const mmf_ekf_model* models, int32_t num_filters, int32_t T
                      const float* mean0, const float* cov0, const float* controls, const float* z,
                      const float* r_tril, float* mean_out, float* cov_out, void* stream);
 
+/* Training forward of the same recursion: mmf_ekf_loop_fwd's arithmetic (bit-identical mean_out / cov_out) that also
+ * records the tape mmf_ekf_loop_bwd needs, pred_out (F,T,N,sd) = mu- and jac_out (F,T,N,sd,sd) = A of every step. */
+int mmf_ekf_loop_train_fwd(const mmf_ekf_model* models, int32_t num_filters, int32_t T, int32_t N,
+                           const float* mean0, const float* cov0, const float* controls, const float* z,
+                           const float* r_tril, float* mean_out, float* cov_out, float* pred_out,
+                           float* jac_out, void* stream);
+
+/* Reverse mode of mmf_ekf_loop_train_fwd with frozen dynamics.  A = df/dx is evaluated at a detached state (A.4),
+ * so it is a constant of the recursion and one step's adjoint is SD x SD algebra given the tape.  Going backwards in
+ * t, with mb / Pb the gradient reaching posterior t (d_means[t] / d_covs[t] plus what step t+1 sent back), P the
+ * posterior covariance of step t-1 (cov0 at t = 0), Pp, S, Sinv = S^-1, Kg recomputed as in the forward, r = z - mu-:
+ *   d_z[t]   = Kg^T mb;                  mb-  = mb - d_z[t]
+ *   Kg_bar   = mb r^T - Pb Pp^T;         S_bar = -Sinv^T Pp^T Kg_bar Sinv^T
+ *   Pp_bar   = (I - Kg)^T Pb + Kg_bar Sinv^T + S_bar
+ *   d_r_tril[t] = (S_bar + S_bar^T) r_tril[t]   (full sd x sd, upper entries included)
+ *   Pb(t-1)  = A^T Pp_bar A;             mb(t-1) = A^T mb-
+ * and d_mean0 = mb(-1), d_cov0 = Pb(-1).  means / covs / pred / jac are the forward's outputs; mean0 and means are
+ * not read (mu- is on the tape) and may be NULL.  d_means and d_covs may each be NULL (= zero).  One thread per
+ * (filter, trajectory), no atomics: the gradients are bit-reproducible run to run.  No workspace. */
+int mmf_ekf_loop_bwd(const mmf_ekf_model* models, int32_t num_filters, int32_t T, int32_t N,
+                     const float* mean0, const float* cov0, const float* z, const float* r_tril,
+                     const float* means, const float* covs, const float* pred, const float* jac,
+                     const float* d_means, const float* d_covs, float* d_mean0, float* d_cov0, float* d_z,
+                     float* d_r_tril, void* stream);
+
 /* Dynamics Jacobian alone (A.4 DynamicsModel.jacobian): states (N,sd), controls (N,cd) ->
  * pred (N,sd), jac (N,sd,sd). */
 int mmf_dynamics_jacobian(const mmf_ekf_model* model, int32_t N, const float* states,

@@ -111,6 +111,12 @@ PROTOTYPES = {
     "mmf_fuse_loglik": (C.c_int, [_i32, _i32, _i32, _vp, _vp, _vp, _vp]),
     "mmf_resample": (C.c_int, [_i32, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp]),
     "mmf_ekf_loop_fwd": (C.c_int, [C.POINTER(EKFModel), _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mmf_ekf_loop_train_fwd": (
+        C.c_int, [C.POINTER(EKFModel), _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mmf_ekf_loop_bwd": (
+        C.c_int,
+        [C.POINTER(EKFModel), _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    ),
     "mmf_dynamics_jacobian": (C.c_int, [C.POINTER(EKFModel), _i32, _vp, _vp, _vp, _vp, _vp]),
     "mmf_kf_fuse_crossmodal": (C.c_int, [_i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mmf_pf_forward_loop_persistent": (C.c_int, [_i32, _i32]),

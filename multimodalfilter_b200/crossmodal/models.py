@@ -15,7 +15,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from .. import fused, ops
+from .. import fused, ops, training
 from ..encoders import ImageEncoder
 from ..fannypack.nn import resblocks
 from ..fannypack.utils import SliceWrapper
@@ -488,6 +488,18 @@ class _MultiFilter(tf_base.Filter, _EnabledModels):
         self.filter_models = nn.ModuleList(filter_models)
         self._enabled_models = [True] * len(self.filter_models)
         self.weighted_covariances = None
+        self.fused_train = True  # training with frozen dynamics: the F filters' recursion and its backward as one kernel each
+
+    @property
+    def fused_train(self):
+        return self.__dict__.get("_mmf_fused_train", True)
+
+    @fused_train.setter
+    def fused_train(self, on):
+        # the member filters follow, so that the step-by-step path (forward) agrees with forward_loop
+        self.__dict__["_mmf_fused_train"] = bool(on)
+        for f in self.filter_models:
+            f.fused_train = bool(on)
 
     @property
     def state_covariance_estimate(self):
@@ -528,8 +540,32 @@ class _MultiFilter(tf_base.Filter, _EnabledModels):
             f._belief_mean, f._belief_covariance = means[i, -1], covs[i, -1]
         return means, covs
 
+    def _train_fused(self, filters, controls, observations):
+        return all(f._initialized for f in filters) and training.fused_ekf_train_applicable(
+            self, filters, self._plan(filters), controls, observations,
+            [t for f in filters for t in (f._belief_mean, f._belief_covariance)])
+
+    def _advance_train(self, filters, controls, z, r_tril):
+        """``_advance`` with autograd (``training.FusedEKFLoop``): the new beliefs keep their ``grad_fn``."""
+        mean0 = torch.stack([f._belief_mean for f in filters])
+        cov0 = torch.stack([f._belief_covariance for f in filters])
+        means, covs = training.FusedEKFLoop.apply(self._plan(filters), mean0, cov0, controls, z, r_tril)
+        for i, f in enumerate(filters):
+            f._belief_mean, f._belief_covariance = means[i, -1], covs[i, -1]
+        return means, covs
+
+    def _sense_sequence_train(self, filters, observations, T, N):
+        zr = [f.sense_sequence(observations, T, N, grad=True) for f in filters]
+        return torch.stack([a[0] for a in zr]), torch.stack([a[1] for a in zr])
+
     def calculate_unimodal_states(self, observations, controls):
         filters = self._enabled_filters()
+        if self._train_fused(filters, controls, observations):
+            zr = [f.virtual_sensor_model(observations=observations) for f in filters]
+            z = torch.stack([a[0] for a in zr])[:, None]
+            r = torch.stack([a[1] for a in zr])[:, None]
+            means, covs = self._advance_train(filters, controls[None], z, r)
+            return means[:, 0], covs[:, 0]
         if self._fusable(filters, controls):
             zr = [f.virtual_sensor_model(observations=observations) for f in filters]
             z = torch.stack([a[0].detach() for a in zr])[:, None]
@@ -582,14 +618,14 @@ class CrossmodalKalmanFilter(_MultiFilter):
             f.states_covariance_prev = cov
         return mean
 
-    def _sequence_weights(self, observations, T, N, device):
-        """(T, K_enabled, N, sd) fusion weights for a whole sequence."""
+    def _sequence_weights(self, observations, T, N, device, grad=False):
+        """(T, K_enabled, N, sd) fusion weights for a whole sequence; ``grad``: with autograd."""
         on = self._enabled_models
         if np.sum(on) < len(on):
             w = _mask_weights(on, N, self.state_dim, device)[on]
             return w[None].expand(T, *w.shape)
         wm = self.crossmodal_weight_model
-        with torch.no_grad():
+        with torch.set_grad_enabled(grad):
             if hasattr(wm, "forward_sequence"):
                 return wm.forward_sequence(observations, T, N)
             obs = SliceWrapper(observations)
@@ -597,6 +633,16 @@ class CrossmodalKalmanFilter(_MultiFilter):
 
     def forward_loop(self, *, observations, controls):
         filters = self._enabled_filters()
+        if isinstance(observations, dict) and self._train_fused(filters, controls, observations):
+            # the F filters in one FusedEKFLoop; the (tiny) fusion stays torch expressions under autograd
+            T, N = controls.shape[:2]
+            assert SliceWrapper(observations).shape[:2] == (T, N)
+            means, covs = self._advance_train(filters, controls, *self._sense_sequence_train(filters, observations, T, N))
+            beta = self._sequence_weights(observations, T, N, controls.device, grad=True)
+            beta = self._blackout_adjust(beta, observations).transpose(0, 1)  # (F,T,N,sd)
+            cw = beta[..., None] * beta[..., None, :]
+            self.weighted_covariances = torch.sum(cw * covs, dim=0)[-1]
+            return weighted_average(means, beta)
         if not self._fusable(filters, controls) or tf_filters._has_hooks(self) or not isinstance(observations, dict):
             return super().forward_loop(observations=observations, controls=controls)
         T, N = controls.shape[:2]
@@ -621,6 +667,12 @@ class CrossmodalKalmanFilter(_MultiFilter):
         self.initialize_beliefs(mean=mean, covariance=cov)
 
 
+def _information_fusion(states, covs):  # ref: base_models/unimodal_kf.py:199-242 (+1e-9 is elementwise)
+    precision = torch.inverse(covs + 1e-9)
+    cov = torch.inverse(precision.sum(dim=0) + 1e-9)
+    return (cov @ (precision @ states[..., None]).sum(dim=0)).squeeze(-1)
+
+
 class UnimodalKalmanFilter(_MultiFilter):
     """ref: crossmodal/base_models/unimodal_kf.py:118-270."""
 
@@ -632,14 +684,17 @@ class UnimodalKalmanFilter(_MultiFilter):
         if states.is_cuda and not (torch.is_grad_enabled() and (states.requires_grad or covs.requires_grad)):
             mean, _ = ops.kf_fuse_unimodal(states, covs)
         else:
-            precision = torch.inverse(covs + 1e-9)
-            cov = torch.inverse(precision.sum(dim=0) + 1e-9)
-            mean = (cov @ (precision @ states[..., None]).sum(dim=0)).squeeze(-1)
+            mean = _information_fusion(states, covs)
         assert mean.shape == (N, self.state_dim)
         return mean
 
     def forward_loop(self, *, observations, controls):
         filters = self._enabled_filters()
+        if isinstance(observations, dict) and self._train_fused(filters, controls, observations):
+            T, N = controls.shape[:2]
+            assert SliceWrapper(observations).shape[:2] == (T, N)
+            means, covs = self._advance_train(filters, controls, *self._sense_sequence_train(filters, observations, T, N))
+            return means[0] if means.shape[0] == 1 else _information_fusion(means, covs)
         if not self._fusable(filters, controls) or tf_filters._has_hooks(self) or not isinstance(observations, dict):
             return super().forward_loop(observations=observations, controls=controls)
         T, N = controls.shape[:2]

@@ -266,6 +266,47 @@ int mmf_ekf_loop_fwd(const mmf_ekf_model* models, int32_t num_filters, int32_t T
   return launch_ekf(P, models[0].state_dim, (cudaStream_t)stream);
 }
 
+int mmf_ekf_loop_train_fwd(const mmf_ekf_model* models, int32_t num_filters, int32_t T, int32_t N, const float* mean0,
+                           const float* cov0, const float* controls, const float* z, const float* r_tril,
+                           float* mean_out, float* cov_out, float* pred_out, float* jac_out, void* stream) {
+  EkfParams P;
+  memset(&P, 0, sizeof(P));
+  int rc = fill_ekf(P, models, num_filters);
+  if (rc) return rc;
+  MMF_REQUIRE(T >= 0 && N >= 0, "ekf_train: bad shape T=%d N=%d", T, N);
+  if (T == 0 || N == 0) return MMF_OK;
+  MMF_REQUIRE(mean0 && cov0 && controls && z && r_tril && mean_out && cov_out && pred_out && jac_out,
+              "ekf_train: NULL buffer");
+  P.T = T; P.N = N; P.jac_only = 0;
+  P.mean0 = mean0; P.cov0 = cov0; P.controls = controls; P.z = z; P.r_tril = r_tril;
+  P.mean_out = mean_out; P.cov_out = cov_out; P.pred_out = pred_out; P.jac_out = jac_out;
+  return launch_ekf(P, models[0].state_dim, (cudaStream_t)stream, /*tape=*/true);
+}
+
+int mmf_ekf_loop_bwd(const mmf_ekf_model* models, int32_t num_filters, int32_t T, int32_t N, const float* mean0,
+                     const float* cov0, const float* z, const float* r_tril, const float* means, const float* covs,
+                     const float* pred, const float* jac, const float* d_means, const float* d_covs, float* d_mean0,
+                     float* d_cov0, float* d_z, float* d_r_tril, void* stream) {
+  (void)mean0;  // mu- of every step is on the tape: the posterior means are not read
+  (void)means;
+  EkfParams F;
+  memset(&F, 0, sizeof(F));
+  int rc = fill_ekf(F, models, num_filters);
+  if (rc) return rc;
+  MMF_REQUIRE(T >= 0 && N >= 0, "ekf_bwd: bad shape T=%d N=%d", T, N);
+  if (N == 0) return MMF_OK;
+  MMF_REQUIRE(cov0 && d_mean0 && d_cov0, "ekf_bwd: NULL buffer");
+  MMF_REQUIRE(T == 0 || (z && r_tril && covs && pred && jac && d_z && d_r_tril), "ekf_bwd: NULL buffer");
+  EkfBwdParams P;
+  memset(&P, 0, sizeof(P));
+  memcpy(P.q, F.q, sizeof(P.q));
+  P.F = num_filters; P.T = T; P.N = N;
+  P.cov0 = cov0; P.z = z; P.r_tril = r_tril; P.covs = covs; P.pred = pred; P.jac = jac;
+  P.d_means = d_means; P.d_covs = d_covs;
+  P.d_mean0 = d_mean0; P.d_cov0 = d_cov0; P.d_z = d_z; P.d_r_tril = d_r_tril;
+  return launch_ekf_bwd(P, models[0].state_dim, (cudaStream_t)stream);
+}
+
 int mmf_dynamics_jacobian(const mmf_ekf_model* model, int32_t N, const float* states, const float* controls,
                           float* pred_out, float* jac_out, void* stream) {
   EkfParams P;

@@ -58,6 +58,67 @@ __device__ __forceinline__ void invert(const float (&A)[SD][SD], float (&inv)[SD
   }
 }
 
+// Q Q^T of one filter's process-noise factor (row-major SD x SD in q).
+template <int SD>
+__device__ __forceinline__ void ekf_qqt(const float* q, float (&Q)[SD][SD]) {
+#pragma unroll
+  for (int i = 0; i < SD; ++i)
+#pragma unroll
+    for (int j = 0; j < SD; ++j) {
+      float s = 0.0f;
+#pragma unroll
+      for (int k = 0; k < SD; ++k) s = fmaf(q[i * SD + k], q[j * SD + k], s);
+      Q[i][j] = s;
+    }
+}
+
+// The covariance half of one EKF step, shared by the forward (k_ekf_loop) and its reverse mode (k_ekf_loop_bwd),
+// which recomputes these from the stored posteriors and the tape instead of saving them:
+//   Pp = A Pm A^T + Q Q^T;  S = Pp + Rt Rt^T;  Sinv = S^-1;  Kg = Pp Sinv
+template <int SD>
+__device__ __forceinline__ void ekf_gain(const float (&A)[SD][SD], const float (&Pm)[SD][SD], const float (&Q)[SD][SD],
+                                         const float (&Rt)[SD][SD], float (&Pp)[SD][SD], float (&Sinv)[SD][SD],
+                                         float (&Kg)[SD][SD]) {
+  float AP[SD][SD], S[SD][SD];
+#pragma unroll
+  for (int i = 0; i < SD; ++i)
+#pragma unroll
+    for (int j = 0; j < SD; ++j) {
+      float s = 0.0f;
+#pragma unroll
+      for (int k = 0; k < SD; ++k) s = fmaf(A[i][k], Pm[k][j], s);
+      AP[i][j] = s;
+    }
+#pragma unroll
+  for (int i = 0; i < SD; ++i)
+#pragma unroll
+    for (int j = 0; j < SD; ++j) {
+      float s = 0.0f;
+#pragma unroll
+      for (int k = 0; k < SD; ++k) s = fmaf(AP[i][k], A[j][k], s);
+      Pp[i][j] = s + Q[i][j];
+    }
+#pragma unroll
+  for (int i = 0; i < SD; ++i)
+#pragma unroll
+    for (int j = 0; j < SD; ++j) {
+      float s = 0.0f;
+#pragma unroll
+      for (int k = 0; k < SD; ++k) s = fmaf(Rt[i][k], Rt[j][k], s);
+      S[i][j] = Pp[i][j] + s;
+    }
+  invert<SD>(S, Sinv);
+#pragma unroll
+  for (int i = 0; i < SD; ++i)
+#pragma unroll
+    for (int j = 0; j < SD; ++j) {
+      float s = 0.0f;
+#pragma unroll
+      for (int k = 0; k < SD; ++k) s = fmaf(Pp[i][k], Sinv[k][j], s);
+      Kg[i][j] = s;
+    }
+}
+
 // One 64x64 layer for R rows held in shared memory.  Lane computes outputs `lane` and `lane+32`.
 // mode: 0 = first half of a resblock (bias, relu), 1 = second half (bias + residual rows, relu),
 //       2 = mid layer (rowbias given in `bias`, relu optional)
@@ -210,7 +271,9 @@ int launch_traj_rows(const mmf_pf_model* model, int N, const float* controls, co
 }
 
 // ---- EKF loop ------------------------------------------------------------------------------------------
-template <int SD>
+// TAPE: also record mu- (pred_out) and A (jac_out) of every step for k_ekf_loop_bwd.  The arithmetic is the same
+// with and without it, so both instantiations produce the same posteriors bit for bit.
+template <int SD, bool TAPE>
 __global__ void __launch_bounds__(EKF_MAX_WARPS * 32, 1) k_ekf_loop(const __grid_constant__ EkfParams P, int wpc) {
   constexpr int R = 1 + SD;
   extern __shared__ __align__(16) float sm[];
@@ -238,15 +301,7 @@ __global__ void __launch_bounds__(EKF_MAX_WARPS * 32, 1) k_ekf_loop(const __grid
 
   const int N = P.N, T = P.T;
   float Q[SD][SD];  // Q Q^T
-#pragma unroll
-  for (int i = 0; i < SD; ++i)
-#pragma unroll
-    for (int j = 0; j < SD; ++j) {
-      float s = 0.0f;
-#pragma unroll
-      for (int k = 0; k < SD; ++k) s = fmaf(P.q[f][i * SD + k], P.q[f][j * SD + k], s);
-      Q[i][j] = s;
-    }
+  ekf_qqt<SD>(P.q[f], Q);
 
   for (int n = blockIdx.x * wpc + wid; n < N && wid < wpc; n += gridDim.x * wpc) {
     float mu[SD], Pm[SD][SD];
@@ -342,54 +397,26 @@ __global__ void __launch_bounds__(EKF_MAX_WARPS * 32, 1) k_ekf_loop(const __grid
         }
         continue;
       }
-      // ---- predict covariance ----------------------------------------------------------------------------
-      float AP[SD][SD], Pp[SD][SD];
-#pragma unroll
-      for (int i = 0; i < SD; ++i)
-#pragma unroll
-        for (int j = 0; j < SD; ++j) {
-          float s = 0.0f;
-#pragma unroll
-          for (int k = 0; k < SD; ++k) s = fmaf(A[i][k], Pm[k][j], s);
-          AP[i][j] = s;
-        }
-#pragma unroll
-      for (int i = 0; i < SD; ++i)
-#pragma unroll
-        for (int j = 0; j < SD; ++j) {
-          float s = 0.0f;
-#pragma unroll
-          for (int k = 0; k < SD; ++k) s = fmaf(AP[i][k], A[j][k], s);
-          Pp[i][j] = s + Q[i][j];
-        }
-      // ---- update (C = I) -----------------------------------------------------------------------------------
+      // ---- predict covariance, update (C = I) -----------------------------------------------------------------
       const size_t ft = ((size_t)f * T + t) * N + n;
-      float Rt[SD][SD], S[SD][SD], Sinv[SD][SD], Kg[SD][SD], zt[SD];
+      float Rt[SD][SD], Pp[SD][SD], Sinv[SD][SD], Kg[SD][SD], zt[SD];
 #pragma unroll
       for (int i = 0; i < SD; ++i) {
         zt[i] = P.z[ft * SD + i];
 #pragma unroll
         for (int j = 0; j < SD; ++j) Rt[i][j] = P.r_tril[(ft * SD + i) * SD + j];
       }
+      if constexpr (TAPE) {
+        if (lane == 0) {
 #pragma unroll
-      for (int i = 0; i < SD; ++i)
+          for (int i = 0; i < SD; ++i) {
+            P.pred_out[ft * SD + i] = pred[i];
 #pragma unroll
-        for (int j = 0; j < SD; ++j) {
-          float s = 0.0f;
-#pragma unroll
-          for (int k = 0; k < SD; ++k) s = fmaf(Rt[i][k], Rt[j][k], s);
-          S[i][j] = Pp[i][j] + s;
+            for (int j = 0; j < SD; ++j) P.jac_out[(ft * SD + i) * SD + j] = A[i][j];
+          }
         }
-      invert<SD>(S, Sinv);
-#pragma unroll
-      for (int i = 0; i < SD; ++i)
-#pragma unroll
-        for (int j = 0; j < SD; ++j) {
-          float s = 0.0f;
-#pragma unroll
-          for (int k = 0; k < SD; ++k) s = fmaf(Pp[i][k], Sinv[k][j], s);
-          Kg[i][j] = s;
-        }
+      }
+      ekf_gain<SD>(A, Pm, Q, Rt, Pp, Sinv, Kg);
 #pragma unroll
       for (int i = 0; i < SD; ++i) {
         float s = 0.0f;
@@ -418,7 +445,7 @@ __global__ void __launch_bounds__(EKF_MAX_WARPS * 32, 1) k_ekf_loop(const __grid
   }
 }
 
-template <int SD>
+template <int SD, bool TAPE>
 static int launch_ekf_sd(const EkfParams& P, cudaStream_t stream) {
   int dev = 0, sms = 148;
   MMF_CUDA(cudaGetDevice(&dev));
@@ -433,7 +460,7 @@ static int launch_ekf_sd(const EkfParams& P, cudaStream_t stream) {
   static thread_local int configured_dev = -1;
   static thread_local size_t window = 0;
   if (configured_dev != dev) {
-    int rc = opt_in_shared_memory(k_ekf_loop<SD>, &window);
+    int rc = opt_in_shared_memory(k_ekf_loop<SD, TAPE>, &window);
     if (rc) return rc;
     configured_dev = dev;
   }
@@ -447,20 +474,194 @@ static int launch_ekf_sd(const EkfParams& P, cudaStream_t stream) {
   const int max_ctas = (sms + P.F - 1) / P.F > 0 ? (sms / P.F > 0 ? sms / P.F : 1) : 1;
   if (ctas > max_ctas) ctas = max_ctas;
   dim3 grid(ctas, P.F);
-  k_ekf_loop<SD><<<grid, wpc * 32, smem, stream>>>(P, wpc);
+  k_ekf_loop<SD, TAPE><<<grid, wpc * 32, smem, stream>>>(P, wpc);
   MMF_LAUNCH_CHECK("k_ekf_loop");
   return MMF_OK;
 }
 
-int launch_ekf(const EkfParams& P, int sd, cudaStream_t stream) {
+int launch_ekf(const EkfParams& P, int sd, cudaStream_t stream, bool tape) {
   switch (sd) {
-    case 1: return launch_ekf_sd<1>(P, stream);
-    case 2: return launch_ekf_sd<2>(P, stream);
-    case 3: return launch_ekf_sd<3>(P, stream);
-    case 4: return launch_ekf_sd<4>(P, stream);
+    case 1: return tape ? launch_ekf_sd<1, true>(P, stream) : launch_ekf_sd<1, false>(P, stream);
+    case 2: return tape ? launch_ekf_sd<2, true>(P, stream) : launch_ekf_sd<2, false>(P, stream);
+    case 3: return tape ? launch_ekf_sd<3, true>(P, stream) : launch_ekf_sd<3, false>(P, stream);
+    case 4: return tape ? launch_ekf_sd<4, true>(P, stream) : launch_ekf_sd<4, false>(P, stream);
   }
   set_error("ekf: state_dim %d unsupported (1..%d)", sd, MMF_MAX_SD);
   return MMF_E_INVALID;
+}
+
+// ---- reverse mode of the EKF loop: one thread per (filter, trajectory), t = T-1 ... 0 in registers ---------------
+// The dynamics Jacobian A is a constant of the recursion (the reference differentiates f at a detached state, A.4) and
+// the dynamics are frozen, so one step's adjoint is SD x SD algebra given A and mu- from the tape.  With mb / Pb the
+// gradient reaching posterior t (the caller's d_means[t] / d_covs[t] plus what step t+1 sent back), r = z - mu-:
+//   z_bar  = Kg^T mb;                       mb-  = mb - z_bar
+//   Kg_bar = mb r^T - Pb Pp^T;              S_bar = -Sinv^T Pp^T Kg_bar Sinv^T
+//   Pp_bar = (I - Kg)^T Pb + Kg_bar Sinv^T + S_bar;    R_bar = (S_bar + S_bar^T) Rt
+//   Pb(t-1) = A^T Pp_bar A;                 mb(t-1) = A^T mb-
+// Every output element is written by exactly one thread: no atomics, bit-reproducible.
+template <int SD>
+__global__ void __launch_bounds__(128) k_ekf_loop_bwd(const __grid_constant__ EkfBwdParams P) {
+  const int N = P.N, T = P.T;
+  const long long total = (long long)P.F * N;
+  for (long long item = blockIdx.x * (long long)blockDim.x + threadIdx.x; item < total;
+       item += (long long)gridDim.x * blockDim.x) {
+    const int f = (int)(item / N), n = (int)(item % N);
+    float Q[SD][SD];
+    ekf_qqt<SD>(P.q[f], Q);
+    float mb[SD], Pb[SD][SD];
+#pragma unroll
+    for (int i = 0; i < SD; ++i) {
+      mb[i] = 0.0f;
+#pragma unroll
+      for (int j = 0; j < SD; ++j) Pb[i][j] = 0.0f;
+    }
+    for (int t = T - 1; t >= 0; --t) {
+      const size_t ft = ((size_t)f * T + t) * N + n;
+      const float* prev = t > 0 ? P.covs + (ft - N) * SD * SD : P.cov0 + ((size_t)f * N + n) * SD * SD;
+      float A[SD][SD], Pm[SD][SD], Rt[SD][SD], r[SD];
+#pragma unroll
+      for (int i = 0; i < SD; ++i) {
+        r[i] = P.z[ft * SD + i] - P.pred[ft * SD + i];
+#pragma unroll
+        for (int j = 0; j < SD; ++j) {
+          A[i][j] = P.jac[(ft * SD + i) * SD + j];
+          Pm[i][j] = prev[i * SD + j];
+          Rt[i][j] = P.r_tril[(ft * SD + i) * SD + j];
+        }
+      }
+      float Pp[SD][SD], Sinv[SD][SD], Kg[SD][SD];
+      ekf_gain<SD>(A, Pm, Q, Rt, Pp, Sinv, Kg);
+      if (P.d_means != nullptr) {
+#pragma unroll
+        for (int i = 0; i < SD; ++i) mb[i] += P.d_means[ft * SD + i];
+      }
+      if (P.d_covs != nullptr) {
+#pragma unroll
+        for (int i = 0; i < SD; ++i)
+#pragma unroll
+          for (int j = 0; j < SD; ++j) Pb[i][j] += P.d_covs[(ft * SD + i) * SD + j];
+      }
+      // z_bar, mb-
+      float mbp[SD];
+#pragma unroll
+      for (int i = 0; i < SD; ++i) {
+        float s = 0.0f;
+#pragma unroll
+        for (int k = 0; k < SD; ++k) s = fmaf(Kg[k][i], mb[k], s);
+        P.d_z[ft * SD + i] = s;
+        mbp[i] = mb[i] - s;
+      }
+      // Kg_bar = mb r^T - Pb Pp^T
+      float Kb[SD][SD];
+#pragma unroll
+      for (int i = 0; i < SD; ++i)
+#pragma unroll
+        for (int j = 0; j < SD; ++j) {
+          float s = 0.0f;
+#pragma unroll
+          for (int k = 0; k < SD; ++k) s = fmaf(Pb[i][k], Pp[j][k], s);
+          Kb[i][j] = mb[i] * r[j] - s;
+        }
+      // S_bar = -Sinv^T (Pp^T Kg_bar) Sinv^T
+      float M1[SD][SD], M2[SD][SD], Sb[SD][SD];
+#pragma unroll
+      for (int i = 0; i < SD; ++i)
+#pragma unroll
+        for (int j = 0; j < SD; ++j) {
+          float s = 0.0f;
+#pragma unroll
+          for (int k = 0; k < SD; ++k) s = fmaf(Pp[k][i], Kb[k][j], s);
+          M1[i][j] = s;
+        }
+#pragma unroll
+      for (int i = 0; i < SD; ++i)
+#pragma unroll
+        for (int j = 0; j < SD; ++j) {
+          float s = 0.0f;
+#pragma unroll
+          for (int k = 0; k < SD; ++k) s = fmaf(Sinv[k][i], M1[k][j], s);
+          M2[i][j] = s;
+        }
+#pragma unroll
+      for (int i = 0; i < SD; ++i)
+#pragma unroll
+        for (int j = 0; j < SD; ++j) {
+          float s = 0.0f;
+#pragma unroll
+          for (int k = 0; k < SD; ++k) s = fmaf(M2[i][k], Sinv[j][k], s);
+          Sb[i][j] = -s;
+        }
+      // R_bar = (S_bar + S_bar^T) Rt: every entry, the upper ones included (as autograd of r_tril @ r_tril^T)
+#pragma unroll
+      for (int i = 0; i < SD; ++i)
+#pragma unroll
+        for (int j = 0; j < SD; ++j) {
+          float s = 0.0f;
+#pragma unroll
+          for (int k = 0; k < SD; ++k) s = fmaf(Sb[i][k] + Sb[k][i], Rt[k][j], s);
+          P.d_r_tril[(ft * SD + i) * SD + j] = s;
+        }
+      // Pp_bar = (I - Kg)^T Pb + Kg_bar Sinv^T + S_bar   (into M1)
+#pragma unroll
+      for (int i = 0; i < SD; ++i)
+#pragma unroll
+        for (int j = 0; j < SD; ++j) {
+          float s = Sb[i][j];
+#pragma unroll
+          for (int k = 0; k < SD; ++k) s = fmaf(((k == i) ? 1.0f : 0.0f) - Kg[k][i], Pb[k][j], s);
+#pragma unroll
+          for (int k = 0; k < SD; ++k) s = fmaf(Kb[i][k], Sinv[j][k], s);
+          M1[i][j] = s;
+        }
+      // Pb <- A^T Pp_bar A,  mb <- A^T mb-
+#pragma unroll
+      for (int i = 0; i < SD; ++i)
+#pragma unroll
+        for (int j = 0; j < SD; ++j) {
+          float s = 0.0f;
+#pragma unroll
+          for (int k = 0; k < SD; ++k) s = fmaf(A[k][i], M1[k][j], s);
+          M2[i][j] = s;
+        }
+#pragma unroll
+      for (int i = 0; i < SD; ++i) {
+        float s = 0.0f;
+#pragma unroll
+        for (int k = 0; k < SD; ++k) s = fmaf(A[k][i], mbp[k], s);
+        mb[i] = s;
+#pragma unroll
+        for (int j = 0; j < SD; ++j) {
+          float u = 0.0f;
+#pragma unroll
+          for (int k = 0; k < SD; ++k) u = fmaf(M2[i][k], A[k][j], u);
+          Pb[i][j] = u;
+        }
+      }
+    }
+    const size_t fn = (size_t)f * N + n;
+#pragma unroll
+    for (int i = 0; i < SD; ++i) {
+      P.d_mean0[fn * SD + i] = mb[i];
+#pragma unroll
+      for (int j = 0; j < SD; ++j) P.d_cov0[(fn * SD + i) * SD + j] = Pb[i][j];
+    }
+  }
+}
+
+int launch_ekf_bwd(const EkfBwdParams& P, int sd, cudaStream_t stream) {
+  const long long total = (long long)P.F * P.N;
+  if (total == 0) return MMF_OK;
+  long long blocks = (total + 127) / 128;
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  switch (sd) {
+    case 1: k_ekf_loop_bwd<1><<<(int)blocks, 128, 0, stream>>>(P); break;
+    case 2: k_ekf_loop_bwd<2><<<(int)blocks, 128, 0, stream>>>(P); break;
+    case 3: k_ekf_loop_bwd<3><<<(int)blocks, 128, 0, stream>>>(P); break;
+    case 4: k_ekf_loop_bwd<4><<<(int)blocks, 128, 0, stream>>>(P); break;
+    default: set_error("ekf_bwd: state_dim %d unsupported (1..%d)", sd, MMF_MAX_SD); return MMF_E_INVALID;
+  }
+  MMF_LAUNCH_CHECK("k_ekf_loop_bwd");
+  return MMF_OK;
 }
 
 // ---- R10 / R11 fusion: one thread per (t, n) row ---------------------------------------------------------

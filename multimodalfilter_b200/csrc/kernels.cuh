@@ -36,6 +36,26 @@ struct EkfParams {
   const float* r_tril;    // (F, T, N, sd, sd)
   float* mean_out;        // (F, T, N, sd)      [jac_only: pred (N, sd)]
   float* cov_out;         // (F, T, N, sd, sd)  [jac_only: jacobian (N, sd, sd)]
+  float* pred_out;        // (F, T, N, sd)      tape: mu- of every step   (launch_ekf(..., tape = true) only)
+  float* jac_out;         // (F, T, N, sd, sd)  tape: A of every step
+};
+
+// Reverse mode of the EKF recursion (k_ekf_loop_bwd); d_means / d_covs may be NULL (= zero).
+struct EkfBwdParams {
+  float q[EKF_MAX_FILTERS][MMF_MAX_SD * MMF_MAX_SD];
+  int F, T, N;
+  const float* cov0;      // (F, N, sd, sd)
+  const float* z;         // (F, T, N, sd)
+  const float* r_tril;    // (F, T, N, sd, sd)
+  const float* covs;      // (F, T, N, sd, sd)  posteriors of the forward
+  const float* pred;      // (F, T, N, sd)      tape
+  const float* jac;       // (F, T, N, sd, sd)  tape
+  const float* d_means;   // (F, T, N, sd)
+  const float* d_covs;    // (F, T, N, sd, sd)
+  float* d_mean0;         // (F, N, sd)
+  float* d_cov0;          // (F, N, sd, sd)
+  float* d_z;             // (F, T, N, sd)
+  float* d_r_tril;        // (F, T, N, sd, sd)
 };
 
 int launch_particle_chain_ffma(const mmf_pf_model* model, int N, int M, const float* states_in, const float* eps,
@@ -53,7 +73,8 @@ int launch_pf_init(int N, int M, int sd, const float* mean, const float* cov, co
                    float* logw, cudaStream_t stream);
 int launch_normalize_resample(const ResampleParams& P, void* workspace, cudaStream_t stream);
 size_t resample_workspace_bytes(int N, int M);
-int launch_ekf(const EkfParams& P, int sd, cudaStream_t stream);
+int launch_ekf(const EkfParams& P, int sd, cudaStream_t stream, bool tape = false);
+int launch_ekf_bwd(const EkfBwdParams& P, int sd, cudaStream_t stream);
 int launch_reweight_train(int N, int M, int K, int sd, uint32_t enabled, const float* ll, const float* w, const float* logw_in,
                           const float* states, float* logw_out, float* est_out, const float* d_est, const float* d_logw,
                           float* d_ll, float* d_w, float* d_logw_in, bool backward, cudaStream_t stream);

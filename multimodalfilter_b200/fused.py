@@ -391,6 +391,11 @@ class EKFPlan:
         self.refresh(z.device)
         return ops.ekf_loop(self.structs, mean0, cov0, controls, z, r_tril)
 
+    def loop_train(self, mean0, cov0, controls, z, r_tril):
+        """``loop`` plus the tape of the backward: -> means, covs, pred (F,T,N,sd), jac (F,T,N,sd,sd)."""
+        self.refresh(z.device)
+        return ops.ekf_loop_train(self.structs, mean0, cov0, controls, z, r_tril)
+
     def jacobian(self, which, states, controls):
         self.refresh(states.device)
         return ops.dynamics_jacobian(self.structs[which], states, controls)

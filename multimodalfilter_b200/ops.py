@@ -492,6 +492,56 @@ def ekf_loop(model_structs, mean0, cov0, controls, z, r_tril):
     return means, covs
 
 
+def ekf_loop_train(model_structs, mean0, cov0, controls, z, r_tril):
+    """``ekf_loop`` that also records the tape of ``ekf_loop_bwd``: -> means (F,T,N,sd), covs (F,T,N,sd,sd),
+    pred (F,T,N,sd) = mu- and jac (F,T,N,sd,sd) = A of every step.  means / covs equal ``ekf_loop``'s bit for bit."""
+    lib = _lib.load()
+    F = len(model_structs)
+    arr = (_lib.EKFModel * F)(*model_structs)
+    mean0, cov0, controls, z, r_tril = map(_f32c, (mean0, cov0, controls, z, r_tril))
+    _, T, N, sd = z.shape
+    assert mean0.shape == (F, N, sd) and cov0.shape == (F, N, sd, sd)
+    assert controls.shape[:2] == (T, N) and r_tril.shape == (F, T, N, sd, sd)
+    means = torch.empty((F, T, N, sd), device=z.device, dtype=torch.float32)
+    covs = torch.empty((F, T, N, sd, sd), device=z.device, dtype=torch.float32)
+    pred = torch.empty_like(means)
+    jac = torch.empty_like(covs)
+    _lib.check(
+        PROFILE.run("ekf_loop_train", 1, lib.mmf_ekf_loop_train_fwd, arr, F, T, N, _lib.ptr(mean0), _lib.ptr(cov0),
+                    _lib.ptr(controls), _lib.ptr(z), _lib.ptr(r_tril), _lib.ptr(means), _lib.ptr(covs), _lib.ptr(pred),
+                    _lib.ptr(jac), _lib.stream_of(z))
+    )
+    return means, covs, pred, jac
+
+
+def ekf_loop_bwd(model_structs, cov0, z, r_tril, covs, pred, jac, d_means=None, d_covs=None):
+    """Reverse mode of ``ekf_loop_train`` (frozen dynamics, A a constant of the recursion): the forward's inputs and
+    outputs plus d_means (F,T,N,sd) | None, d_covs (F,T,N,sd,sd) | None -> d_mean0, d_cov0, d_z, d_r_tril."""
+    lib = _lib.load()
+    F = len(model_structs)
+    arr = (_lib.EKFModel * F)(*model_structs)
+    cov0, z, r_tril, covs, pred, jac = map(_f32c, (cov0, z, r_tril, covs, pred, jac))
+    _, T, N, sd = z.shape
+    assert cov0.shape == (F, N, sd, sd) and r_tril.shape == covs.shape == jac.shape == (F, T, N, sd, sd)
+    assert pred.shape == z.shape
+    d_means = None if d_means is None else _f32c(d_means)
+    d_covs = None if d_covs is None else _f32c(d_covs)
+    assert d_means is None or d_means.shape == z.shape
+    assert d_covs is None or d_covs.shape == covs.shape
+    dev = z.device
+    d_mean0 = torch.empty((F, N, sd), device=dev, dtype=torch.float32)
+    d_cov0 = torch.empty_like(cov0)
+    d_z = torch.empty_like(z)
+    d_r = torch.empty_like(r_tril)
+    _lib.check(
+        PROFILE.run("ekf_loop_bwd", 1, lib.mmf_ekf_loop_bwd, arr, F, T, N, None, _lib.ptr(cov0), _lib.ptr(z),
+                    _lib.ptr(r_tril), None, _lib.ptr(covs), _lib.ptr(pred), _lib.ptr(jac), _lib.ptr(d_means),
+                    _lib.ptr(d_covs), _lib.ptr(d_mean0), _lib.ptr(d_cov0), _lib.ptr(d_z), _lib.ptr(d_r),
+                    _lib.stream_of(z))
+    )
+    return d_mean0, d_cov0, d_z, d_r
+
+
 def dynamics_jacobian(model_struct, states, controls):
     """A.4: states (N,sd), controls (N,cd) -> pred (N,sd), jacobian (N,sd,sd)."""
     lib = _lib.load()

@@ -6,6 +6,8 @@ crossmodal/eval_helpers.py:125-142), executing in the sm_100a kernels of ``libmm
 Dispatch (SURVEY.md section 8b):
   * recognised architectures (the reference's gated-residual dynamics and per-particle heads,
     see ``fused.py``) and no autograd  -> fully fused kernels, observation encoders hoisted over T;
+  * training with frozen recognised dynamics -> the particle filter's ``training.FusedHeads`` / ``Reweight``, the
+    Kalman filters' ``training.FusedEKFLoop`` (the recursion and its backward as one kernel each);
   * anything else (user-defined modules, or gradients required) -> the modules run as torch
     modules on the GPU and only the reweight / normalise / estimate / resample stages run in the
     kernels (torch ops where a gradient has to flow).
@@ -549,6 +551,7 @@ class VirtualSensorExtendedKalmanFilter(ExtendedKalmanFilter):
             measurement_model=_IdentityMeasurementModel(state_dim=dynamics_model.state_dim),
         )
         self.virtual_sensor_model = virtual_sensor_model
+        self.fused_train = True  # training with frozen dynamics: the recursion and its backward as one kernel each
 
     def fused_plan(self):
         cached = self.__dict__.get("_mmf_plan")
@@ -564,10 +567,25 @@ class VirtualSensorExtendedKalmanFilter(ExtendedKalmanFilter):
             and not _needs_grad(self, self._belief_mean, self._belief_covariance)
         )
 
+    def _train_fused(self, observations, controls):
+        return self._initialized and training.fused_ekf_train_applicable(
+            self, [self], self.fused_plan(), controls, observations, (self._belief_mean, self._belief_covariance))
+
+    def _advance_train(self, controls, z, r_tril):
+        """Training step(s) through ``training.FusedEKFLoop``: controls (T,N,cd), z (T,N,sd), r_tril (T,N,sd,sd) ->
+        posterior means (T,N,sd).  The new belief keeps its ``grad_fn``, so the next call chains the gradient."""
+        means, covs = training.FusedEKFLoop.apply(self.fused_plan(), self._belief_mean[None], self._belief_covariance[None],
+                                                  controls, z[None], r_tril[None])
+        self._belief_mean, self._belief_covariance = means[0, -1], covs[0, -1]
+        return means[0]
+
     def forward(self, *, observations, controls):
         assert self._initialized, "Kalman filter not initialized: call initialize_beliefs() first"
         require_cuda(self._belief_mean, "the belief mean")
         z, r_tril = self.virtual_sensor_model(observations=observations)
+        if self._train_fused(observations, controls):
+            assert controls.shape[0] == self._belief_mean.shape[0]
+            return self._advance_train(controls[None], z[None], r_tril[None])[0]
         if not self._use_fused(controls):
             self.measurement_model.scale_tril = r_tril
             return super().forward(observations=z, controls=controls)
@@ -579,10 +597,10 @@ class VirtualSensorExtendedKalmanFilter(ExtendedKalmanFilter):
         self._belief_mean, self._belief_covariance = means[0, 0], covs[0, 0]
         return self._belief_mean
 
-    def sense_sequence(self, observations, T, N):
-        """Virtual-sensor outputs for all T steps: z (T,N,sd), r_tril (T,N,sd,sd)."""
+    def sense_sequence(self, observations, T, N, grad=False):
+        """Virtual-sensor outputs for all T steps: z (T,N,sd), r_tril (T,N,sd,sd); ``grad``: with autograd."""
         vs = self.virtual_sensor_model
-        with torch.no_grad():
+        with torch.set_grad_enabled(grad):
             if type(vs).__name__ in TIME_BATCHABLE or getattr(vs, "_mmf_time_batchable", False):
                 outs = fused.batched_over_time(lambda o: vs(observations=o), observations, T, N)
                 z = torch.cat([o[0] for o in outs]).reshape(T, N, -1)
@@ -595,6 +613,11 @@ class VirtualSensorExtendedKalmanFilter(ExtendedKalmanFilter):
         return z.contiguous(), r.contiguous()
 
     def forward_loop(self, *, observations, controls):
+        if isinstance(observations, dict) and self._train_fused(observations, controls):
+            T, N = controls.shape[:2]
+            assert SliceWrapper(observations).shape[:2] == (T, N), "observations and controls disagree on (T, N)"
+            z, r_tril = self.sense_sequence(observations, T, N, grad=True)
+            return self._advance_train(controls, z, r_tril)
         if not self._initialized or not self._use_fused(controls) or _has_hooks(self) or not isinstance(observations, dict):
             return super().forward_loop(observations=observations, controls=controls)
         require_cuda(controls, "controls")

@@ -1,4 +1,5 @@
-"""BPTT support: the fused training step of the particle filter (BASELINE config C4).
+"""BPTT support: the fused training step of the particle filter (BASELINE config C4), and ``FusedEKFLoop``, the
+extended Kalman filters' recursion and its reverse mode in one launch each.
 
 In train mode torchfilter does not resample (A.3) and every curriculum of the reference freezes the
 dynamics before end-to-end training (ref: scripts/push_task/train_push.py:154,213), so the particle
@@ -179,6 +180,60 @@ class Reweight(torch.autograd.Function):
         modw = rest[0] if ctx.has_modw else None
         d_ll, d_w, d_in = ops.pf_reweight_train_bwd(ll, modw, logw_in, states, ctx.mask, d_est, d_logw)
         return d_ll, d_w, d_in, None, None
+
+
+class FusedEKFLoop(torch.autograd.Function):
+    """(plan, mean0 (F,N,sd), cov0 (F,N,sd,sd), controls (T,N,cd), z (F,T,N,sd), r_tril (F,T,N,sd,sd)) -> (means
+    (F,T,N,sd), covs (F,T,N,sd,sd)): F extended Kalman filters over T steps in one launch (``mmf_ekf_loop_train_fwd``),
+    and the reverse mode in one more (``mmf_ekf_loop_bwd``), which returns the gradients of mean0, cov0, z and r_tril.
+
+    The dynamics are frozen and the reference evaluates their Jacobian A at a detached state (A.4), so A carries no
+    gradient and the backward is SD x SD algebra given A and mu- of every step: the forward records both (the tape)
+    instead of the backward re-running the dynamics MLP.  The controls receive no gradient (the dynamics are frozen
+    and the controls are data)."""
+
+    @staticmethod
+    def forward(ctx, plan, mean0, cov0, controls, z, r_tril):
+        cov0, z, r_tril = cov0.detach().contiguous(), z.detach().contiguous(), r_tril.detach().contiguous()
+        means, covs, pred, jac = plan.loop_train(mean0.detach().contiguous(), cov0, controls.detach(), z, r_tril)
+        # the structs (q_tril) and the weight buffers they point at, as of this forward
+        ctx.structs, ctx.buffers = plan.structs, plan._buffers
+        ctx.save_for_backward(cov0, z, r_tril, covs, pred, jac)
+        ctx.set_materialize_grads(False)
+        return means, covs
+
+    @staticmethod
+    def backward(ctx, d_means, d_covs):
+        if d_means is None and d_covs is None:
+            return None, None, None, None, None, None
+        cov0, z, r_tril, covs, pred, jac = ctx.saved_tensors
+        d_mean0, d_cov0, d_z, d_r = ops.ekf_loop_bwd(ctx.structs, cov0, z, r_tril, covs, pred, jac, d_means, d_covs)
+        return None, d_mean0, d_cov0, None, d_z, d_r
+
+
+def ekf_train_structure_ok(owner, filters, plan) -> bool:
+    """The checks of ``fused_ekf_train_applicable`` that need no device: a recognised plan, ``owner.fused_train``, no
+    hooks anywhere in ``owner`` (the fused step never calls the dynamics modules) and frozen dynamics in every filter
+    (gradients into the dynamics MLP are not part of the kernels' adjoint)."""
+    if plan is None or not getattr(owner, "fused_train", True):
+        return False
+    if any(m._forward_hooks or m._forward_pre_hooks for m in owner.modules()):
+        return False
+    return not any(p.requires_grad for f in filters for p in f.dynamics_model.parameters())
+
+
+def fused_ekf_train_applicable(owner, filters, plan, controls, observations, beliefs) -> bool:
+    """Train the EKF recursion of ``filters`` (the enabled filters of ``owner``) through ``FusedEKFLoop``: a gradient
+    is needed (grad mode on, and a parameter of ``owner`` or one of the ``beliefs`` requires it), the structural checks
+    of ``ekf_train_structure_ok`` pass, and controls and observations are CUDA fp32 tensors."""
+    if not torch.is_grad_enabled():
+        return False
+    if not (any(t is not None and t.requires_grad for t in beliefs) or any(p.requires_grad for p in owner.parameters())):
+        return False
+    if not ekf_train_structure_ok(owner, filters, plan):
+        return False
+    tensors = [controls, *(observations.values() if isinstance(observations, dict) else [observations])]
+    return all(isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float32 for t in tensors)
 
 
 def fused_train_applicable(filt, plan, resample: bool) -> bool:
