@@ -54,12 +54,12 @@ class RecordedNoise:
 
     def init_eps(self, M, N, sd, like):
         assert self._init.shape == (M, N, sd)
-        return self._init.to(like.dtype)
+        return self._init.to(device=like.device, dtype=like.dtype)
 
     def process_eps(self, rows, sd, like):
         eps = self._eps.pop(0)
         assert eps.shape == (rows, sd)
-        return eps.to(like.dtype)
+        return eps.to(device=like.device, dtype=like.dtype)
 
     def resample_indices(self, probs, S, logits=None):
         u = self._u.pop(0)

@@ -26,6 +26,8 @@ import torch
 from multimodalfilter_b200 import ops
 from oracle import pinned
 
+from util import kernel_ran as _kernel_ran
+
 DEV = "cuda:0"
 MODES = ["multinomial", "multinomial_fast", "systematic", "systematic_fast"]
 ONE_MINUS = 1.0 - 2.0 ** -53  # the largest double below 1
@@ -195,17 +197,6 @@ def test_tie_constructor_flips_the_pinned_index():
 
 
 # ---- GPU helpers ------------------------------------------------------------------------------------------------------
-def _kernel_ran(names, want):
-    """`want` is a kernel as the profiler demangles it, e.g. k_normalize_resample<false,32> (spaces ignored); the mangled
-    spelling (k_normalize_resampleILb0ELi32EE) is accepted too."""
-    base, _, args = want.partition("<")
-    mangled = base
-    if args:
-        code = {"false": "Lb0E", "true": "Lb1E"}
-        mangled += "I" + "".join(code.get(a, f"Li{a}E") for a in args.rstrip(">").split(",")) + "E"
-    return any(want in n.replace(" ", "") or mangled in n for n in names)
-
-
 def profiled(fn, want):
     """Run fn under torch.profiler and assert that the kernel `want` ran and no resampling kernel of another path did."""
     from torch.profiler import ProfilerActivity, profile

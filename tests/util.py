@@ -63,6 +63,17 @@ def assert_close(actual, expected, rtol=1e-4, atol=None, msg=""):
     )
 
 
+def kernel_ran(names, want):
+    """`want` is a kernel as the profiler demangles it, e.g. k_normalize_resample<false,32> (spaces ignored); the mangled
+    spelling (k_normalize_resampleILb0ELi32EE) is accepted too."""
+    base, _, args = want.partition("<")
+    mangled = base
+    if args:
+        code = {"false": "Lb0E", "true": "Lb1E"}
+        mangled += "I" + "".join(code.get(a, f"Li{a}E") for a in args.rstrip(">").split(",")) + "E"
+    return any(want in n.replace(" ", "") or mangled in n for n in names)
+
+
 def header_symbols():
     text = open(os.path.join(REPO, "include", "mmf_b200.h")).read()
     text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
