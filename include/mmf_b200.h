@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MMF_ABI_VERSION 2
+#define MMF_ABI_VERSION 3
 #define MMF_UNITS 64
 #define MMF_MAX_SD 4
 #define MMF_MAX_CD 16
@@ -296,28 +296,26 @@ int mmf_pf_heads_backward(const mmf_pf_model* model, int32_t N, int32_t M, const
                           uint32_t enabled_mask, float* delta_out, void* stream);
 /* ---- image observation encoder: convolutional trunk (SURVEY.md 8(f)-1) ------------------------------------
  * Replaces the Conv2d layers of observation_image_layers (ref: crossmodal/push_models/layers.py:93-101,
- * crossmodal/door_models/layers.py:43-57) for 32x32 single-channel images.  Activation maps are bf16 hi/lo
- * planes, mmf_enc_map_bytes(channels) bytes per image, and MUST be zero-initialised once by the caller (the
- * kernels rely on zero guard regions they never write).
- *   mmf_enc_stem      Conv2d(1, 32, 5, padding=2) + ReLU; w = weight as [tap 25][32] then bias[32], fp32.
- *   mmf_enc_conv3x3   Conv2d(cin, cout, 3, padding=1) [+ residual map] [+ ReLU] on the tensor cores
- *                     (bf16 hi/lo split operands, fp32 accumulation); (cin, cout) in {(32,32), (32,16), (16,<=16)}.
- *                     w_image = bf16 [tap 9][cin/8][2 npad rows: hi then lo][8] then fp32 bias[npad], npad = 32
- *                     if cout > 16 else 16 (rows >= cout zero).  Writes out_map (planes, npad channels) and/or out_nchw
- *                     (n_images, cout, 32, 32) fp32. */
-size_t mmf_enc_map_bytes(int32_t channels);
-/*   mmf_enc_trunk     the whole trunk (stem, residual block, 32->16, 16->cout) of every image in ONE launch: a
- *                     persistent CTA carries an image through all layers, its activation maps live in `scratch`
- *                     (mmf_enc_trunk_scratch_bytes() bytes, zero-initialised once by the caller; stays L2-resident).
- *                     weights = [w_image block1 | w_image block2 | w_image 32->16 | w_image 16->cout | stem w],
- *                     each as described above (mmf_enc_trunk_weight_bytes() bytes in total). */
+ * crossmodal/door_models/layers.py:43-57) for 32x32 single-channel images:
+ *   x = relu(stem(image)), t = relu(block1(x)), y = relu(block2(t) + x), z = relu(conv3(y)), out = conv4(z)
+ * with stem = Conv2d(1, 32, 5, padding=2), block1, block2 = Conv2d(32, 32, 3, padding=1),
+ * conv3 = Conv2d(32, 16, 3, padding=1), conv4 = Conv2d(16, cout, 3, padding=1), cout <= 16.
+ *   mmf_enc_trunk     the whole trunk of every image in ONE launch: a persistent CTA carries an image through all
+ *                     layers, the 3x3 layers on the tensor cores (bf16 hi/lo split operands, fp32 accumulation).  Its
+ *                     activation maps live in `scratch` (mmf_enc_trunk_scratch_bytes() bytes, stays L2-resident), which
+ *                     MUST be zero-initialised once by the caller: the kernel relies on zero guard regions it never writes.
+ *                     out_nchw = (n_images, cout, 32, 32) fp32.
+ *                     weights = [w_image block1 | w_image block2 | w_image conv3 | w_image conv4 | stem w]
+ *                     (mmf_enc_trunk_weight_bytes() bytes in total), where
+ *                     w_image of a Conv2d(cin, c, 3) = bf16 [tap 9][cin/8][2 npad rows: hi then lo][8] then fp32
+ *                       bias[npad], npad = 32 if c > 16 else 16: row n, element j of (tap, chunk k) holds
+ *                       weight[n][8k + j][tap / 3][tap % 3] split as hi = rn_bf16(w), lo = rn_bf16(w - hi); rows >= c
+ *                       and bias entries >= c are zero;
+ *                     stem w = fp32 weight as [tap 25][32] (element [5 ky + kx][c] = weight[c][0][ky][kx]) then bias[32]. */
 size_t mmf_enc_trunk_scratch_bytes(void);
 size_t mmf_enc_trunk_weight_bytes(void);
 int mmf_enc_trunk(int32_t n_images, int32_t cout, const float* images, const void* weights, void* scratch,
                   float* out_nchw, void* stream);
-int mmf_enc_stem(int32_t n_images, const float* images, const float* w, void* out_map, void* stream);
-int mmf_enc_conv3x3(int32_t n_images, int32_t cin, int32_t cout, const void* in_map, const void* w_image,
-                    const void* res_map, int32_t relu, void* out_map, float* out_nchw, void* stream);
 
 /* Parameter gradients of the heads from the saved activations and the deltas (both (K, L+1, 16, rows, 4)
  * chunk-major planes: element [k][l][c][p][j] = column 4c+j of row p), fp32 reductions over the N*M rows:

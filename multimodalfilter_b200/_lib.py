@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmmf_b200.so")
 
 MAX_SD, MAX_CD, MAX_HEADS, UNITS = 4, 16, 4, 64
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 RESAMPLE_NONE = 0
 RESAMPLE_MULTINOMIAL_STRICT = 1
@@ -129,12 +129,9 @@ PROTOTYPES = {
     "mmf_pf_heads_backward": (C.c_int, [C.POINTER(PFModel), _i32, _i32, _vp, _vp, _u32, _vp, _vp]),
     "mmf_pf_heads_weight_grads_workspace_bytes": (_sz, [_i32, _i32, C.c_int64]),
     "mmf_pf_heads_weight_grads": (C.c_int, [_i32, _i32, C.c_int64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
-    "mmf_enc_map_bytes": (_sz, [_i32]),
     "mmf_enc_trunk_scratch_bytes": (_sz, []),
     "mmf_enc_trunk_weight_bytes": (_sz, []),
     "mmf_enc_trunk": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp]),
-    "mmf_enc_stem": (C.c_int, [_i32, _vp, _vp, _vp, _vp]),
-    "mmf_enc_conv3x3": (C.c_int, [_i32, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp]),
     "mmf_pf_reweight_train_fwd": (C.c_int, [_i32, _i32, _i32, _i32, C.c_uint32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mmf_pf_reweight_train_bwd": (C.c_int, [_i32, _i32, _i32, _i32, C.c_uint32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mmf_row_mlp": (

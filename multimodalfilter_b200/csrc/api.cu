@@ -436,25 +436,6 @@ int mmf_row_mlp(int64_t rows, const mmf_mlp_op* ops, int32_t n_ops, const float*
                         n_outputs, scratch_floats, (cudaStream_t)stream);
 }
 
-size_t mmf_enc_map_bytes(int32_t channels) { return enc_map_bytes_host(channels); }
-
-int mmf_enc_stem(int32_t n_images, const float* images, const float* w, void* out_map, void* stream) {
-  MMF_REQUIRE(n_images >= 0, "enc_stem: negative image count");
-  MMF_REQUIRE(n_images == 0 || (images && w && out_map), "enc_stem: NULL buffer");
-  MMF_REQUIRE(((uintptr_t)out_map & 15) == 0, "enc_stem: map must be 16-byte aligned");
-  return launch_enc_stem(n_images, images, w, out_map, (cudaStream_t)stream);
-}
-
-int mmf_enc_conv3x3(int32_t n_images, int32_t cin, int32_t cout, const void* in_map, const void* w_image,
-                    const void* res_map, int32_t relu, void* out_map, float* out_nchw, void* stream) {
-  MMF_REQUIRE(n_images >= 0, "enc_conv3x3: negative image count");
-  MMF_REQUIRE(n_images == 0 || (in_map && w_image), "enc_conv3x3: NULL input");
-  MMF_REQUIRE(out_map || out_nchw, "enc_conv3x3: no output requested");
-  MMF_REQUIRE((((uintptr_t)in_map | (uintptr_t)w_image | (uintptr_t)res_map | (uintptr_t)out_map) & 15) == 0,
-              "enc_conv3x3: maps and the operand image must be 16-byte aligned");
-  return launch_enc_conv3x3(n_images, cin, cout, in_map, w_image, res_map, relu, out_map, out_nchw, (cudaStream_t)stream);
-}
-
 size_t mmf_enc_trunk_scratch_bytes(void) { return enc_trunk_scratch_bytes(); }
 size_t mmf_enc_trunk_weight_bytes(void) { return enc_trunk_weight_bytes(); }
 

@@ -89,59 +89,6 @@ __device__ __forceinline__ void unpack8(const uint4& hi4, const uint4& lo4, floa
 }
 __device__ __forceinline__ bool enc_valid(int pos) { return pos < ENC_NPOS && (pos % ENC_PITCH) < 32; }
 
-// ---- 5x5 stem on the CUDA cores: image (32x32 fp32) -> 32-channel map, ReLU --------------------------------
-// weights: w[25][32] (tap-major) then bias[32], fp32.
-__global__ void __launch_bounds__(256) k_enc_stem(const float* __restrict__ images, const float* __restrict__ w,
-                                                  uint8_t* __restrict__ out_map, int n_images) {
-  __shared__ float img[36 * 36];
-  __shared__ __align__(16) float ws[25 * 32 + 32];
-  for (int i = threadIdx.x; i < 25 * 32 + 32; i += blockDim.x) ws[i] = w[i];
-  for (int image = blockIdx.x; image < n_images; image += gridDim.x) {
-    __syncthreads();
-    for (int i = threadIdx.x; i < 36 * 36; i += blockDim.x) {
-      const int y = i / 36 - 2, x = i % 36 - 2;
-      img[i] = (y >= 0 && y < 32 && x >= 0 && x < 32) ? images[(size_t)image * 1024 + y * 32 + x] : 0.0f;
-    }
-    __syncthreads();
-    uint8_t* map = out_map + (size_t)image * enc_map_bytes(32);
-    for (int pos = threadIdx.x; pos < ENC_TILES * 128; pos += blockDim.x) {
-      const bool valid = enc_valid(pos);
-      float acc[32];
-      if (valid) {
-        const int y = pos / ENC_PITCH, x = pos % ENC_PITCH;
-#pragma unroll
-        for (int c = 0; c < 32; ++c) acc[c] = ws[25 * 32 + c];
-        for (int ky = 0; ky < 5; ++ky) {
-#pragma unroll
-          for (int kx = 0; kx < 5; ++kx) {
-            const float p = img[(y + ky) * 36 + x + kx];
-            const float4* w4 = reinterpret_cast<const float4*>(ws + (ky * 5 + kx) * 32);
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-              const float4 t = w4[q];
-              acc[4 * q] = fmaf(t.x, p, acc[4 * q]);
-              acc[4 * q + 1] = fmaf(t.y, p, acc[4 * q + 1]);
-              acc[4 * q + 2] = fmaf(t.z, p, acc[4 * q + 2]);
-              acc[4 * q + 3] = fmaf(t.w, p, acc[4 * q + 3]);
-            }
-          }
-        }
-      }
-#pragma unroll
-      for (int kc = 0; kc < 4; ++kc) {
-        float v[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) v[j] = valid ? fmaxf(acc[kc * 8 + j], 0.0f) : 0.0f;
-        uint4 hi4, lo4;
-        split8(v, hi4, lo4);
-        uint8_t* plane = map + (size_t)(kc * 2) * ENC_PLANE_B + (size_t)(ENC_GUARD + pos) * 16;
-        *reinterpret_cast<uint4*>(plane) = hi4;
-        *reinterpret_cast<uint4*>(plane + ENC_PLANE_B) = lo4;
-      }
-    }
-  }
-}
-
 // this thread's accumulator row: columns [0, NPAD) hold hi*hi + lo*hi, [NPAD, 2 NPAD) hold hi*lo -> their sum
 template <int NPAD>
 __device__ __forceinline__ void load_accumulator(uint32_t taddr, uint32_t (&d)[NPAD]) {
@@ -182,194 +129,8 @@ __device__ __forceinline__ void issue_conv(uint32_t st_addr, uint32_t w_addr, ui
   }
 }
 
-// ---- 3x3 convolution as implicit GEMM on tcgen05 -----------------------------------------------------------
-struct ConvParams {
-  const uint8_t* in_map;    // CIN channels
-  const uint8_t* w_image;   // [tap 9][chunk CIN/8][2 NPAD rows: hi then lo][8] bf16, then bias fp32[NPAD]
-  const uint8_t* res_map;   // residual input (same channel count as the output) or null
-  uint8_t* out_map;         // bf16 hi/lo planes of NPAD channels, or null
-  float* out_nchw;          // (n_images, cout, 32, 32) fp32, or null
-  int n_images, cout, relu;
-};
-
-template <int CIN, int NPAD>
-__global__ void __launch_bounds__(ENC_THREADS, 1) k_enc_conv3x3(const __grid_constant__ ConvParams P) {
-  constexpr int KC = CIN / 8;                     // 16-byte channel chunks
-  constexpr int PLANES = KC * 2;
-  constexpr int STAGE_B = PLANES * ENC_WIN_B;
-  constexpr int W_B = 2 * 9 * KC * NPAD * 16;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* w_s = smem;                                         // W_B bytes + bias
-  float* bias_s = reinterpret_cast<float*>(smem + W_B);
-  uint8_t* stage0 = smem + ((W_B + NPAD * 4 + 127) & ~127);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(stage0 + ENC_STAGES * STAGE_B);
-  uint64_t* full = bars;                      // TMA bytes landed            (producer -> issuer)
-  uint64_t* mma_done = bars + ENC_STAGES;     // accumulator complete        (issuer -> epilogue)
-  uint64_t* stage_free = bars + 2 * ENC_STAGES;  // MMAs have read the stage   (issuer -> producer)
-  uint64_t* tmem_free = bars + 3 * ENC_STAGES;   // epilogue has read D        (epilogue -> issuer)
-  uint64_t* wbar = bars + 4 * ENC_STAGES;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(wbar + 1);
-
-  const int tid = threadIdx.x;
-  const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
-  if (tid == 0) {
-    for (int s = 0; s < ENC_STAGES; ++s) {
-      mbar_init(full + s, 1);
-      mbar_init(mma_done + s, 1);
-      mbar_init(stage_free + s, 1);
-      mbar_init(tmem_free + s, 4);
-    }
-    mbar_init(wbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(ENC_STAGES * ENC_DCOLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  const long long items = (long long)P.n_images * ENC_TILES;
-  const long long first = blockIdx.x, step = gridDim.x;
-
-  if (warp == 0) {
-    // ------------------------------------------------------------------------------------------ TMA producer
-    if (elect_one_sync()) {
-      mbar_expect_tx(wbar, W_B + NPAD * 4);
-      for (uint32_t off = 0; off < (uint32_t)(W_B + NPAD * 4); off += 32768) {
-        const uint32_t n = (uint32_t)(W_B + NPAD * 4) - off < 32768 ? (uint32_t)(W_B + NPAD * 4) - off : 32768;
-        bulk_g2s(w_s + off, P.w_image + off, n, wbar);
-      }
-      long long i = 0;
-      for (long long w = first; w < items; w += step, ++i) {
-        const int s = (int)(i % ENC_STAGES);
-        const uint32_t par = (uint32_t)((i / ENC_STAGES) & 1);
-        mbar_wait(stage_free + s, par ^ 1u);
-        const long long image = w / ENC_TILES;
-        const int tile = (int)(w % ENC_TILES);
-        const uint8_t* src = P.in_map + (size_t)image * enc_map_bytes(CIN) + (size_t)(ENC_GUARD + tile * 128 - ENC_HALO) * 16;
-        mbar_expect_tx(full + s, STAGE_B);
-#pragma unroll
-        for (int pl = 0; pl < PLANES; ++pl)
-          bulk_g2s(stage0 + s * STAGE_B + pl * ENC_WIN_B, src + (size_t)pl * ENC_PLANE_B, ENC_WIN_B, full + s);
-      }
-    }
-    __syncwarp();
-  } else if (warp == 1) {
-    // -------------------------------------------------------------------------------------------- MMA issuer
-    mbar_wait(wbar, 0);
-    if (elect_one_sync()) {
-      const uint32_t w_addr = smem_u32(w_s);
-      long long i = 0;
-      for (long long w = first; w < items; w += step, ++i) {
-        const int s = (int)(i % ENC_STAGES);
-        const uint32_t par = (uint32_t)((i / ENC_STAGES) & 1);
-        mbar_wait(tmem_free + s, par ^ 1u);
-        mbar_wait(full + s, par);
-        tc_fence_after();
-        const uint32_t st_addr = smem_u32(stage0 + s * STAGE_B);
-        const uint32_t d = tmem_base + s * ENC_DCOLS;
-        issue_conv<CIN, NPAD>(st_addr, w_addr, d);
-        tc_commit(mma_done + s);
-        tc_commit(stage_free + s);
-      }
-    }
-    __syncwarp();
-  } else if (warp >= 4) {
-    // ------------------------------------------------------------------------------------- epilogue groups
-    const int eg = (warp - 4) >> 2;                 // group 0 handles even items, group 1 odd items
-    const int quad = warp & 3;
-    const int r = quad * 32 + (tid & 31);           // row of the tile == TMEM lane
-    mbar_wait(wbar, 0);                             // bias is in shared memory
-    long long i = 0;
-    for (long long w = first; w < items; w += step, ++i) {
-      if ((int)(i & 1) != eg) continue;
-      const int s = (int)(i % ENC_STAGES);
-      const uint32_t par = (uint32_t)((i / ENC_STAGES) & 1);
-      const long long image = w / ENC_TILES;
-      const int pos = (int)(w % ENC_TILES) * 128 + r;
-      const bool valid = enc_valid(pos);
-      mbar_wait(mma_done + s, par);
-      tc_fence_after();
-      uint32_t d[NPAD];
-      const uint32_t taddr = tmem_base + s * ENC_DCOLS + ((uint32_t)(quad * 32) << 16);
-      load_accumulator<NPAD>(taddr, d);
-      tc_fence_before();
-      __syncwarp();
-      if ((tid & 31) == 0) mbar_arrive(tmem_free + s);  // D[s] may be overwritten by the item after next
-
-      const size_t plane_off = (size_t)(ENC_GUARD + pos) * 16;
-#pragma unroll
-      for (int kc = 0; kc < NPAD / 8; ++kc) {
-        float v[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) v[j] = __uint_as_float(d[kc * 8 + j]) + bias_s[kc * 8 + j];
-        if (P.res_map != nullptr) {
-          const uint8_t* rp = P.res_map + (size_t)image * enc_map_bytes(NPAD) + (size_t)(kc * 2) * ENC_PLANE_B + plane_off;
-          float x[8];
-          unpack8(__ldg(reinterpret_cast<const uint4*>(rp)), __ldg(reinterpret_cast<const uint4*>(rp + ENC_PLANE_B)), x);
-#pragma unroll
-          for (int j = 0; j < 8; ++j) v[j] += x[j];
-        }
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          if (P.relu) v[j] = fmaxf(v[j], 0.0f);
-          if (!valid) v[j] = 0.0f;
-        }
-        if (P.out_map != nullptr) {
-          uint4 hi4, lo4;
-          split8(v, hi4, lo4);
-          uint8_t* op = P.out_map + (size_t)image * enc_map_bytes(NPAD) + (size_t)(kc * 2) * ENC_PLANE_B + plane_off;
-          *reinterpret_cast<uint4*>(op) = hi4;
-          *reinterpret_cast<uint4*>(op + ENC_PLANE_B) = lo4;
-        }
-        if (P.out_nchw != nullptr && valid) {
-          const int y = pos / ENC_PITCH, x = pos % ENC_PITCH;
-#pragma unroll
-          for (int j = 0; j < 8; ++j)
-            if (kc * 8 + j < P.cout) P.out_nchw[(((size_t)image * P.cout + kc * 8 + j) * 32 + y) * 32 + x] = v[j];
-        }
-      }
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(ENC_STAGES * ENC_DCOLS) : "memory");
-  }
-}
-
-template <int CIN, int NPAD>
-static int launch_conv(const ConvParams& P, cudaStream_t stream) {
-  constexpr int W_B = 2 * 9 * (CIN / 8) * NPAD * 16;
-  constexpr int STAGE_B = (CIN / 8) * 2 * ENC_WIN_B;
-  const size_t smem = ((W_B + NPAD * 4 + 127) & ~127) + (size_t)ENC_STAGES * STAGE_B + 256;
-  static thread_local int configured_dev = -1;
-  static thread_local size_t window = 0;
-  int dev = 0, sms = 148;
-  MMF_CUDA(cudaGetDevice(&dev));
-  MMF_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  if (configured_dev != dev) {
-    int rc = opt_in_shared_memory(k_enc_conv3x3<CIN, NPAD>, &window);
-    if (rc) return rc;
-    configured_dev = dev;
-  }
-  MMF_REQUIRE(smem <= window, "conv3x3 needs %zu B of shared memory (window %zu B)", smem, window);
-  long long grid = (long long)P.n_images * ENC_TILES;
-  if (grid > sms) grid = sms;
-  k_enc_conv3x3<CIN, NPAD><<<(unsigned)grid, ENC_THREADS, smem, stream>>>(P);
-  MMF_LAUNCH_CHECK("k_enc_conv3x3");
-  return MMF_OK;
-}
-
 // ---- fused trunk: all five layers of one image by one CTA, activation maps in L2-resident scratch ---------------
-// The layer-by-layer kernels above stream every map through HBM (ncu: 3.7 TB/s, 57 % of peak, tensor pipe 26 %).
-// Here a persistent CTA carries an image through stem -> block1 -> block2(+x) -> 32->16 -> 16->8 by itself: its four
+// A persistent CTA carries an image through stem -> block1 -> block2(+x) -> 32->16 -> 16->8 by itself: its four
 // scratch maps (640 KB: x double-buffered, t/z, y) are private, so 148 CTAs keep 95 MB hot in the 126 MB L2 and HBM only
 // sees the raw image and the final (8, 32, 32) activations.  Work items = (layer, tile) in order; tile t of layer l+1 only needs tiles
 // t-1..t+1 of layer l, tracked by one mbarrier per (layer, tile), so the TMA -> MMA -> epilogue ring never drains
@@ -387,7 +148,7 @@ constexpr int TR_SCRATCH_MAPS = 4;            // x (two buffers), t / z, y
 
 struct TrunkParams {
   const float* images;      // (n, 32, 32)
-  const uint8_t* weights;   // [W block1 | W block2 | W 32->16 | W 16->8 | stem fp32], as packed for the layer kernels
+  const uint8_t* weights;   // [W block1 | W block2 | W 32->16 | W 16->8 | stem fp32], layouts in mmf_b200.h
   uint8_t* scratch;         // gridDim.x * TR_SCRATCH_MAPS * enc_map_bytes(32), zero-initialised once
   float* out_nchw;          // (n, cout, 32, 32)
   int n_images, cout;
@@ -641,342 +402,6 @@ __global__ void __launch_bounds__(ENC_THREADS, 1) k_enc_trunk(const __grid_const
   }
 }
 
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&r)[8]) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr)
-               : "memory");
-}
-
-// ---- fused trunk, the three dx taps of a stencil row stacked along N -----------------------------------------------
-// The SS-form MMAs are bound by the shared-memory operand read (A: 8 KB per K step and tap).  The three taps of one
-// stencil ROW (dx = -1, 0, +1) see the same input rows up to a one-position shift, so they can share ONE read of A if
-// the shift is moved to the OUTPUT side: with the weights of the three taps stacked along N,
-//   Y[q][dx][c] = sum_{dy, k} in[q + 34 dy][k] * W[dy][dx][k][c]        (3 A windows instead of 9, N = 3 x 2 Cout)
-//   out[p][c]   = Y[p-1][-1][c] + Y[p][0][c] + Y[p+1][+1][c]           (epilogue: warp shuffles between TMEM lanes)
-// A tile therefore carries 128 rows of Y but owns 126 outputs (rows 1..126); tiles advance by 126 positions.
-// Weight image per layer: [dy 3][chunk Cin/8][6 Cout rows: hi dx-1 | hi dx0 | hi dx+1 | lo dx-1 | lo dx0 | lo dx+1][8];
-// the three split products (hi*hi, hi*lo, lo*hi) are three N = 3 Cout MMAs into the same accumulator columns.
-constexpr int DX_TILE = 126;
-constexpr int DX_DCOLS = 96;   // accumulator columns per slot (3 dx x 32)
-constexpr int DX_THREADS = 640;  // producer, issuer, 2 idle warps, 4 epilogue groups of 4 warps
-
-template <int CIN, int NPAD>
-__device__ __forceinline__ void issue_conv_dx(uint32_t st_addr, uint32_t w_addr, uint32_t d) {
-  constexpr int KC = CIN / 8;
-  constexpr uint32_t IDESC = make_idesc(3 * NPAD, 128);  // three dx taps side by side
-  uint32_t acc = 0;
-#pragma unroll
-  for (int dy = 0; dy < 3; ++dy) {
-    const int shift = ENC_HALO + (dy - 1) * ENC_PITCH;
-#pragma unroll
-    for (int ks = 0; ks < CIN / 16; ++ks) {
-      const uint32_t a_hi = st_addr + (uint32_t)((2 * ks) * 2) * ENC_WIN_B + (uint32_t)shift * 16;
-      const uint32_t a_lo = a_hi + ENC_WIN_B;
-      const uint64_t da_hi = make_desc_interleave(a_hi, 2 * ENC_WIN_B, 128);
-      const uint64_t da_lo = make_desc_interleave(a_lo, 2 * ENC_WIN_B, 128);
-      // rows [0, 3 NPAD) of the (dy, chunk) block = W_hi of the three taps, rows [3 NPAD, 6 NPAD) = W_lo
-      const uint32_t b = w_addr + (uint32_t)((dy * KC + 2 * ks) * 6 * NPAD) * 16;
-      const uint64_t db_hi = make_desc_interleave(b, 6 * NPAD * 16, 128);
-      const uint64_t db_lo = make_desc_interleave(b + 3 * NPAD * 16, 6 * NPAD * 16, 128);
-      // all three split products accumulate into the SAME 3 NPAD columns: the accumulator stays 96 columns wide
-      // (four slots in TMEM, epilogue decoupled from the MMAs) at the price of reading A_hi twice
-      mma_ss(d, da_hi, db_hi, IDESC, acc);
-      mma_ss(d, da_hi, db_lo, IDESC, 1);
-      mma_ss(d, da_lo, db_hi, IDESC, 1);
-      acc = 1;
-    }
-  }
-}
-
-template <int NPAD>
-__device__ __forceinline__ void epilogue_dx(uint32_t taddr, float* xch, int quad, int eg, const float* bias_s,
-                                            const uint8_t* res_map, bool relu, bool owner, bool valid, int pos,
-                                            uint8_t* out_map, float* out_img, int cout) {
-  const int lane = threadIdx.x & 31;
-  if (res_map != nullptr && owner) {  // the residual rows are needed at the very end: start fetching them now
-    const uint8_t* rp = res_map + (size_t)(ENC_GUARD + (pos < 0 ? 0 : pos)) * 16;
-#pragma unroll
-    for (int pl = 0; pl < NPAD / 4; ++pl) asm volatile("prefetch.global.L1 [%0];" ::"l"(rp + (size_t)pl * ENC_PLANE_B));
-  }
-  // the dx = -1 and dx = +1 blocks of this row in one go (one wait for all the TMEM loads)
-  uint32_t ym[NPAD], yp[NPAD];
-#pragma unroll
-  for (int c = 0; c < NPAD; c += 16) {
-    tmem_ld16(taddr + c, reinterpret_cast<uint32_t(&)[16]>(ym[c]));
-    tmem_ld16(taddr + 2 * NPAD + c, reinterpret_cast<uint32_t(&)[16]>(yp[c]));
-  }
-  tc_wait_ld();
-  // rows at the warp boundaries travel through shared memory: xch[warp][0] = Y[-1 block] of lane 31 (for the next warp's
-  // lane 0), xch[warp][1] = Y[+1 block] of lane 0 (for the previous warp's lane 31)
-  if (lane == 31) {
-#pragma unroll
-    for (int c = 0; c < NPAD; ++c) xch[quad * 64 + c] = __uint_as_float(ym[c]);
-  }
-  if (lane == 0) {
-#pragma unroll
-    for (int c = 0; c < NPAD; ++c) xch[quad * 64 + 32 + c] = __uint_as_float(yp[c]);
-  }
-  group_bar(1 + eg, 128);
-  const size_t plane_off = (size_t)(ENC_GUARD + (pos < 0 ? 0 : pos)) * 16;
-#pragma unroll
-  for (int kc = 0; kc < NPAD / 8; ++kc) {
-    uint32_t y0[8];
-    tmem_ld8(taddr + NPAD + kc * 8, y0);
-    float v[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      float left = __shfl_up_sync(0xffffffffu, __uint_as_float(ym[kc * 8 + j]), 1);     // Y[p-1][dx = -1]
-      float right = __shfl_down_sync(0xffffffffu, __uint_as_float(yp[kc * 8 + j]), 1);  // Y[p+1][dx = +1]
-      if (lane == 0 && quad > 0) left = xch[(quad - 1) * 64 + kc * 8 + j];
-      if (lane == 31 && quad < 3) right = xch[(quad + 1) * 64 + 32 + kc * 8 + j];
-      v[j] = left + right + bias_s[kc * 8 + j];
-    }
-    tc_wait_ld();
-#pragma unroll
-    for (int j = 0; j < 8; ++j) v[j] += __uint_as_float(y0[j]);
-    if (res_map != nullptr && owner) {
-      const uint8_t* rp = res_map + (size_t)(kc * 2) * ENC_PLANE_B + plane_off;
-      float x[8];
-      unpack8(*reinterpret_cast<const uint4*>(rp), *reinterpret_cast<const uint4*>(rp + ENC_PLANE_B), x);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) v[j] += x[j];
-    }
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      if (relu) v[j] = fmaxf(v[j], 0.0f);
-      if (!valid) v[j] = 0.0f;
-    }
-    if (out_map != nullptr && owner) {
-      uint4 hi4, lo4;
-      split8(v, hi4, lo4);
-      uint8_t* op = out_map + (size_t)(kc * 2) * ENC_PLANE_B + plane_off;
-      *reinterpret_cast<uint4*>(op) = hi4;
-      *reinterpret_cast<uint4*>(op + ENC_PLANE_B) = lo4;
-    }
-    if (out_img != nullptr && valid) {
-      const int y = pos / ENC_PITCH, x = pos % ENC_PITCH;
-#pragma unroll
-      for (int j = 0; j < 8; ++j)
-        if (kc * 8 + j < cout) out_img[((size_t)(kc * 8 + j) * 32 + y) * 32 + x] = v[j];
-    }
-  }
-}
-
-// four epilogue groups (warps 4-19), one per accumulator slot: the epilogue (global stores + release per tile) is
-// latency-bound, the MMA side no longer is
-__global__ void __launch_bounds__(DX_THREADS, 1) k_enc_trunk_dx(const __grid_constant__ TrunkParams P) {
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* w_s = smem;
-  uint8_t* stage0 = smem + ((TR_W_B + 127) & ~127);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(stage0 + ENC_STAGES * TR_STAGE_B);
-  uint64_t* full = bars;
-  uint64_t* mma_done = bars + ENC_STAGES;
-  uint64_t* stage_free = bars + 2 * ENC_STAGES;
-  uint64_t* tmem_free = bars + 3 * ENC_STAGES;
-  uint64_t* wbar = bars + 4 * ENC_STAGES;
-  uint64_t* stem_done = wbar + 1;                  // [x buffer 0|1][tile]: stem output of an image is written and published
-  uint64_t* tile_done = stem_done + 2 * ENC_TILES;  // [layer 1..3][tile]: that tile of the layer's OUTPUT map
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tile_done + 3 * ENC_TILES);
-  // boundary rows exchanged between the warps of an epilogue group: [group][item parity][warp][left|right][32]
-  float* xch = reinterpret_cast<float*>(smem + ((TR_W_B + 127) & ~127) + ENC_STAGES * TR_STAGE_B + 1024);
-
-  const int tid = threadIdx.x;
-  const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
-  if (tid == 0) {
-    for (int s = 0; s < ENC_STAGES; ++s) {
-      mbar_init(full + s, 1);
-      mbar_init(mma_done + s, 1);
-      mbar_init(stage_free + s, 1);
-      mbar_init(tmem_free + s, 4);
-    }
-    for (int i = 0; i < 5 * ENC_TILES; ++i) mbar_init(stem_done + i, 4);
-    mbar_init(wbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  const size_t map32 = enc_map_bytes(32);
-  // x is double-buffered: the stem of image k+1 is computed in the shadow of image k's convolutions
-  uint8_t* sx0 = P.scratch + (size_t)blockIdx.x * TR_SCRATCH_MAPS * map32;
-  uint8_t* st = sx0 + 2 * map32;                              // block1 output, later the 16-channel map z
-  uint8_t* sy = st + map32;                                   // resblock output
-  // shared-memory offsets of the per-layer weights
-  constexpr int OFF_W[5] = {2 * TR_W2_B + TR_W3_B + TR_W4_B, 0, TR_W2_B, 2 * TR_W2_B, 2 * TR_W2_B + TR_W3_B};
-
-  if (warp == 0) {
-    // ------------------------------------------------------------------------------------------ TMA producer
-    if (elect_one_sync()) {
-      mbar_expect_tx(wbar, TR_W_B);
-      for (uint32_t off = 0; off < (uint32_t)TR_W_B; off += 32768) {
-        const uint32_t n = (uint32_t)TR_W_B - off < 32768 ? (uint32_t)TR_W_B - off : 32768;
-        bulk_g2s(w_s + off, P.weights + off, n, wbar);
-      }
-      long long c = 0;
-      int k = 0;
-      for (long long image = blockIdx.x; image < P.n_images; image += gridDim.x, ++k) {
-        const uint32_t ipar = (uint32_t)(k & 1);
-        for (int layer = 1; layer <= 4; ++layer) {
-          const uint8_t* in = layer == 1 ? sx0 + (size_t)(k & 1) * map32 : layer == 2 ? st : layer == 3 ? sy : st;
-          const int planes = layer == 4 ? 4 : 8;
-          for (int tile = 0; tile < ENC_TILES; ++tile, ++c) {
-            const int s = (int)(c % ENC_STAGES);
-            const uint32_t par = (uint32_t)((c / ENC_STAGES) & 1);
-            mbar_wait(stage_free + s, par ^ 1u);
-            // the window reaches into the neighbouring tiles of the producing layer
-            // layer 1 reads the stem output in x[k & 1] (completed once every second image), the others layer - 1
-            uint64_t* dep = layer == 1 ? stem_done + (k & 1) * ENC_TILES : tile_done + (layer - 2) * ENC_TILES;
-            const uint32_t dpar = layer == 1 ? (uint32_t)((k >> 1) & 1) : ipar;
-            // input positions [126 tile - 36, 126 tile + 162]: producer tiles are 128 wide for the stem, 126 otherwise
-            const int lo_pos = tile * DX_TILE - 36, hi_pos = tile * DX_TILE + 162;
-            const int width = layer == 1 ? 128 : DX_TILE;
-            const int t_lo = lo_pos < 0 ? 0 : lo_pos / width;
-            int t_hi = hi_pos / width;
-            if (t_hi > ENC_TILES - 1) t_hi = ENC_TILES - 1;
-            for (int tt = t_lo; tt <= t_hi; ++tt) mbar_wait(dep + tt, dpar);
-            asm volatile("fence.proxy.async.global;" ::: "memory");
-            const uint8_t* src = in + (size_t)(ENC_GUARD + tile * DX_TILE - 1 - ENC_HALO) * 16;
-            mbar_expect_tx(full + s, (uint32_t)planes * ENC_WIN_B);
-            for (int pl = 0; pl < planes; ++pl)
-              bulk_g2s(stage0 + s * TR_STAGE_B + pl * ENC_WIN_B, src + (size_t)pl * ENC_PLANE_B, ENC_WIN_B, full + s);
-          }
-        }
-      }
-    }
-    __syncwarp();
-  } else if (warp == 1) {
-    // -------------------------------------------------------------------------------------------- MMA issuer
-    mbar_wait(wbar, 0);
-    if (elect_one_sync()) {
-      const uint32_t w_addr = smem_u32(w_s);
-      long long c = 0;
-      for (long long image = blockIdx.x; image < P.n_images; image += gridDim.x) {
-        for (int layer = 1; layer <= 4; ++layer) {
-          for (int tile = 0; tile < ENC_TILES; ++tile, ++c) {
-            const int s = (int)(c % ENC_STAGES);
-            const uint32_t par = (uint32_t)((c / ENC_STAGES) & 1);
-            const int slot = s;                                  // accumulator slot == shared-memory stage
-            const uint32_t dpar = par;
-            mbar_wait(tmem_free + slot, dpar ^ 1u);
-            mbar_wait(full + s, par);
-            tc_fence_after();
-            const uint32_t st_addr = smem_u32(stage0 + s * TR_STAGE_B);
-            const uint32_t d = tmem_base + slot * DX_DCOLS;
-            if (layer <= 2) issue_conv_dx<32, 32>(st_addr, w_addr + OFF_W[layer], d);
-            else if (layer == 3) issue_conv_dx<32, 16>(st_addr, w_addr + OFF_W[3], d);
-            else issue_conv_dx<16, 16>(st_addr, w_addr + OFF_W[4], d);
-            tc_commit(mma_done + slot);
-            tc_commit(stage_free + s);
-          }
-        }
-      }
-    }
-    __syncwarp();
-  } else if (warp >= 4) {
-    // ------------------------------------------------------------ epilogue groups (and the stem on the CUDA cores)
-    const int eg = (warp - 4) >> 2;
-    const int quad = warp & 3;
-    const int r = quad * 32 + (tid & 31);
-    mbar_wait(wbar, 0);
-    const float* wstem = reinterpret_cast<const float*>(w_s + OFF_W[0]);
-    // stem tile `tile` of image `img` (the kk-th image of this CTA) -> x[kk & 1]
-    auto stem_tile = [&](long long img, int kk, int tile) {
-      const float* im = P.images + (size_t)img * 1024;
-      uint8_t* sx = sx0 + (size_t)(kk & 1) * map32;
-      const int pos = tile * 128 + r;
-      const bool valid = enc_valid(pos);
-      float acc[32];
-#pragma unroll
-      for (int ch = 0; ch < 32; ++ch) acc[ch] = wstem[25 * 32 + ch];
-      if (valid) {
-        const int y = pos / ENC_PITCH, x = pos % ENC_PITCH;
-        for (int ky = 0; ky < 5; ++ky) {
-          const int yy = y + ky - 2;
-#pragma unroll
-          for (int kx = 0; kx < 5; ++kx) {
-            const int xx = x + kx - 2;
-            const float p = (yy >= 0 && yy < 32 && xx >= 0 && xx < 32) ? __ldg(im + yy * 32 + xx) : 0.0f;
-            const float4* w4 = reinterpret_cast<const float4*>(wstem + (ky * 5 + kx) * 32);
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-              const float4 t = w4[q];
-              acc[4 * q] = fmaf(t.x, p, acc[4 * q]);
-              acc[4 * q + 1] = fmaf(t.y, p, acc[4 * q + 1]);
-              acc[4 * q + 2] = fmaf(t.z, p, acc[4 * q + 2]);
-              acc[4 * q + 3] = fmaf(t.w, p, acc[4 * q + 3]);
-            }
-          }
-        }
-      }
-#pragma unroll
-      for (int kc = 0; kc < 4; ++kc) {
-        float v[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) v[j] = valid ? fmaxf(acc[kc * 8 + j], 0.0f) : 0.0f;
-        uint4 hi4, lo4;
-        split8(v, hi4, lo4);
-        uint8_t* plane = sx + (size_t)(kc * 2) * ENC_PLANE_B + (size_t)(ENC_GUARD + pos) * 16;
-        *reinterpret_cast<uint4*>(plane) = hi4;
-        *reinterpret_cast<uint4*>(plane + ENC_PLANE_B) = lo4;
-      }
-      publish_tile(stem_done + (kk & 1) * ENC_TILES + tile);
-    };
-    // the first image's stem up front; afterwards the stem of image k+1 rides along with the convolution items of
-    // image k (one stem tile every fourth item), where the epilogue warps would otherwise wait for the tensor pipe
-    if ((long long)blockIdx.x < P.n_images)
-      for (int tile = 0; tile < ENC_TILES; ++tile)
-        if ((tile & 3) == eg) stem_tile(blockIdx.x, 0, tile);
-    long long c = 0;
-    int k = 0;
-    for (long long image = blockIdx.x; image < P.n_images; image += gridDim.x, ++k) {
-      const long long next = image + gridDim.x;
-      const uint8_t* sx = sx0 + (size_t)(k & 1) * map32;
-      int j = 0;
-      for (int layer = 1; layer <= 4; ++layer) {
-        for (int tile = 0; tile < ENC_TILES; ++tile, ++c, ++j) {
-          if ((j & 3) == 0 && (j >> 2) < ENC_TILES && next < P.n_images && (((j >> 2) & 3) == eg)) stem_tile(next, k + 1, j >> 2);
-          if ((int)(c & 3) != eg) continue;
-          const int pos = tile * DX_TILE - 1 + r;              // this thread's ROW of Y; it owns output `pos` if 1 <= r <= 126
-          const bool owner = r >= 1 && r <= DX_TILE;
-          const bool valid = owner && pos >= 0 && enc_valid(pos);
-          const int slot = (int)(c % ENC_STAGES);
-          const uint32_t dpar = (uint32_t)((c / ENC_STAGES) & 1);
-          mbar_wait(mma_done + slot, dpar);
-          tc_fence_after();
-          const uint32_t taddr = tmem_base + slot * DX_DCOLS + ((uint32_t)(quad * 32) << 16);
-          float* my_xch = xch + ((size_t)(eg * 2 + (int)((c >> 2) & 1)) * 4) * 64;
-          const float* bias_s = reinterpret_cast<const float*>(
-              w_s + OFF_W[layer] + (layer <= 2 ? TR_W2_B - 128 : layer == 3 ? TR_W3_B - 64 : TR_W4_B - 64));
-          float* out_img = P.out_nchw + (size_t)image * P.cout * 1024;
-          if (layer == 1) epilogue_dx<32>(taddr, my_xch, quad, eg, bias_s, nullptr, true, owner, valid, pos, st, nullptr, 0);
-          else if (layer == 2) epilogue_dx<32>(taddr, my_xch, quad, eg, bias_s, sx, true, owner, valid, pos, sy, nullptr, 0);
-          else if (layer == 3) epilogue_dx<16>(taddr, my_xch, quad, eg, bias_s, nullptr, true, owner, valid, pos, st, nullptr, 0);
-          else epilogue_dx<16>(taddr, my_xch, quad, eg, bias_s, nullptr, false, owner, valid, pos, nullptr, out_img, P.cout);
-          tc_fence_before();
-          __syncwarp();
-          if ((tid & 31) == 0) mbar_arrive(tmem_free + slot);
-          if (layer < 4) publish_tile(tile_done + (layer - 1) * ENC_TILES + tile);
-        }
-      }
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
-}
-
 static int trunk_grid(int* grid_out) {
   int dev = 0, sms = 148;
   MMF_CUDA(cudaGetDevice(&dev));
@@ -1013,61 +438,13 @@ int launch_enc_trunk(int n_images, int cout, const float* images, const void* we
   if (configured_dev != dev) {
     rc = opt_in_shared_memory(k_enc_trunk, &window);
     if (rc) return rc;
-    rc = opt_in_shared_memory(k_enc_trunk_dx, &window);
-    if (rc) return rc;
-    if (rc) return rc;
     configured_dev = dev;
   }
   MMF_REQUIRE(smem <= window, "encoder trunk needs %zu B of shared memory (window %zu B)", smem, window);
   if (grid > n_images) grid = n_images;
-  // MMF_ENC_VARIANT (parity-green, measured per 16,384 images on B200):
-  //   0 = one MMA pair per tap and K step, A windows read from shared memory by the MMAs (default, 5.2 ms)
-  //   3 = the three dx taps of a stencil row stacked along N, the dx shift applied in the epilogue with warp shuffles:
-  //       a third of the A windows and MMAs (with the epilogue body disabled the pipeline runs in 3.7 ms), four epilogue
-  //       groups; as built the epilogue is the limiter and it lands at 4.9 ms, level with variant 0 on the same box
-  // (TS-form variants -- A through a TMEM ring filled by gather warps, 5.5-5.7 ms -- were measured and removed, see
-  //  DESIGN.md section 3.2 and the git history.)
-  static const int variant = [] {  // read once when first used: no getenv on the launch path
-    const char* env = getenv("MMF_ENC_VARIANT");
-    return env ? atoi(env) : 0;
-  }();
-  if (variant == 3) k_enc_trunk_dx<<<grid, DX_THREADS, smem, stream>>>(P);
-  else k_enc_trunk<<<grid, ENC_THREADS, smem, stream>>>(P);
+  k_enc_trunk<<<grid, ENC_THREADS, smem, stream>>>(P);
   MMF_LAUNCH_CHECK("k_enc_trunk");
   return MMF_OK;
-}
-
-size_t enc_map_bytes_host(int channels) { return enc_map_bytes(channels); }
-
-int launch_enc_stem(int n_images, const float* images, const float* w, void* out_map, cudaStream_t stream) {
-  if (n_images == 0) return MMF_OK;
-  int dev = 0, sms = 148;
-  MMF_CUDA(cudaGetDevice(&dev));
-  MMF_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  long long grid = n_images < (long long)sms * 4 ? n_images : (long long)sms * 4;
-  k_enc_stem<<<(unsigned)grid, 256, 0, stream>>>(images, w, static_cast<uint8_t*>(out_map), n_images);
-  MMF_LAUNCH_CHECK("k_enc_stem");
-  return MMF_OK;
-}
-
-int launch_enc_conv3x3(int n_images, int cin, int cout, const void* in_map, const void* w_image, const void* res_map,
-                       int relu, void* out_map, float* out_nchw, cudaStream_t stream) {
-  if (n_images == 0) return MMF_OK;
-  ConvParams P;
-  P.in_map = static_cast<const uint8_t*>(in_map);
-  P.w_image = static_cast<const uint8_t*>(w_image);
-  P.res_map = static_cast<const uint8_t*>(res_map);
-  P.out_map = static_cast<uint8_t*>(out_map);
-  P.out_nchw = out_nchw;
-  P.n_images = n_images;
-  P.cout = cout;
-  P.relu = relu;
-  const int npad = cout <= 16 ? 16 : 32;
-  if (cin == 32 && npad == 32) return launch_conv<32, 32>(P, stream);
-  if (cin == 32 && npad == 16) return launch_conv<32, 16>(P, stream);
-  if (cin == 16 && npad == 16) return launch_conv<16, 16>(P, stream);
-  set_error("conv3x3: unsupported channel counts %d -> %d (supported: 32->32, 32->16, 16->(<=16))", cin, cout);
-  return MMF_E_INVALID;
 }
 
 }  // namespace mmf

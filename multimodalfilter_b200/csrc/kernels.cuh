@@ -97,14 +97,10 @@ size_t heads_dw_workspace_bytes(int K, int L, long long P);
 int launch_heads_dw(int K, int L, long long P, int sd, const float* act, const float* delta, const float* x,
                     const float* d_ll, float* dW, float* db, float* g_in, float* g_out, void* workspace,
                     cudaStream_t stream);
-size_t enc_map_bytes_host(int channels);
 size_t enc_trunk_weight_bytes();
 size_t enc_trunk_scratch_bytes();
 int launch_enc_trunk(int n_images, int cout, const float* images, const void* weights, void* scratch, float* out_nchw,
                      cudaStream_t stream);
-int launch_enc_stem(int n_images, const float* images, const float* w, void* out_map, cudaStream_t stream);
-int launch_enc_conv3x3(int n_images, int cin, int cout, const void* in_map, const void* w_image, const void* res_map,
-                       int relu, void* out_map, float* out_nchw, cudaStream_t stream);
 int launch_row_mlp(long long rows, const mmf_mlp_op* ops, int n_ops, const float* weights, const float* const* inputs,
                    const int32_t* in_dims, const int32_t* in_slots, int n_inputs, float* const* outputs,
                    const int32_t* out_dims, const int32_t* out_slots, int n_outputs, int scratch, cudaStream_t stream);

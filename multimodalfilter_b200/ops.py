@@ -2,7 +2,6 @@
 marshalling.  Every function here launches hand-written sm_100a kernels; none has a torch or CPU
 fallback."""
 import ctypes as C
-import os
 import math
 
 import torch
@@ -172,15 +171,6 @@ def pf_heads_weight_grads(act, delta, states, d_ll):
 
 
 # ---- image encoder trunk ------------------------------------------------------------------------------------
-def enc_map_bytes(channels: int) -> int:
-    return int(_lib.load().mmf_enc_map_bytes(channels))
-
-
-def enc_new_map(n_images: int, channels: int, device) -> torch.Tensor:
-    """Zero-initialised activation map (bf16 hi/lo planes); the zero guards are never written by the kernels."""
-    return torch.zeros(n_images * enc_map_bytes(channels), dtype=torch.uint8, device=device)
-
-
 def enc_pack_stem(conv) -> torch.Tensor:
     """Conv2d(1, 32, 5) -> fp32 [tap 25][32] + bias[32]."""
     w = conv.weight.detach().float().reshape(32, 25).t().contiguous().reshape(-1)
@@ -207,49 +197,11 @@ def enc_pack_conv3x3(conv) -> torch.Tensor:
     return torch.cat([img, bias.view(torch.uint8).reshape(-1)]).contiguous()
 
 
-def enc_stem(images, w_stem, out_map):
-    lib = _lib.load()
-    n = images.shape[0]
-    _lib.check(PROFILE.run("enc_stem", 1, lib.mmf_enc_stem, n, _lib.ptr(images), _lib.ptr(w_stem), _lib.ptr(out_map),
-                           _lib.stream_of(images)))
-
-
-def enc_conv3x3(n_images, cin, cout, in_map, w_image, *, res_map=None, relu=True, out_map=None, out_nchw=None):
-    lib = _lib.load()
-    _lib.check(PROFILE.run("enc_conv3x3", 1, lib.mmf_enc_conv3x3, n_images, cin, cout, _lib.ptr(in_map),
-                           _lib.ptr(w_image), _lib.ptr(res_map), int(relu), _lib.ptr(out_map), _lib.ptr(out_nchw),
-                           _lib.stream_of(in_map)))
-
-
-def enc_pack_conv3x3_dx(conv) -> torch.Tensor:
-    """Conv2d(cin, cout, 3) -> bf16 [dy 3][cin/8][6 npad rows: hi dx-1 | hi dx0 | hi dx+1 | lo dx-1 | lo dx0 | lo dx+1][8]
-    + fp32 bias[npad]: the operand image of the dx-stacked trunk kernel (MMF_ENC_VARIANT=3)."""
-    w = conv.weight.detach().float()
-    cout, cin = w.shape[0], w.shape[1]
-    npad = 32 if cout > 16 else 16
-    wp = torch.zeros(npad, cin, 3, 3, device=w.device)
-    wp[:cout] = w
-    hi = wp.to(torch.bfloat16)
-    lo = (wp - hi.float()).to(torch.bfloat16)
-    t = torch.stack([hi, lo])                                   # (hl, n, c, ky, kx)
-    t = t.reshape(2, npad, cin // 8, 8, 3, 3).permute(4, 2, 0, 5, 1, 3)  # (ky, kc, hl, kx, n, j)
-    img = t.contiguous().view(torch.uint8).reshape(-1)
-    bias = torch.zeros(npad, device=w.device)
-    bias[:cout] = conv.bias.detach().float()
-    return torch.cat([img, bias.view(torch.uint8).reshape(-1)]).contiguous()
-
-
-def enc_trunk_variant() -> int:
-    return int(os.environ.get("MMF_ENC_VARIANT", "0"))
-
-
 def enc_pack_trunk(convs) -> torch.Tensor:
-    """[stem, block1, block2, 32->16, 16->cout] Conv2d modules -> the weight buffer of mmf_enc_trunk (the layout of
-    the 3x3 layers depends on the kernel variant: dx-stacked for variant 3)."""
+    """[stem, block1, block2, 32->16, 16->cout] Conv2d modules -> the weight buffer of mmf_enc_trunk."""
     stem, c2a, c2b, c3, c4 = convs
-    pack = enc_pack_conv3x3_dx if enc_trunk_variant() == 3 else enc_pack_conv3x3
-    buf = torch.cat([pack(c2a), pack(c2b), pack(c3), pack(c4),
-                     enc_pack_stem(stem).view(torch.uint8).reshape(-1)]).contiguous()
+    buf = torch.cat([enc_pack_conv3x3(c) for c in (c2a, c2b, c3, c4)] +
+                    [enc_pack_stem(stem).view(torch.uint8).reshape(-1)]).contiguous()
     assert buf.numel() == int(_lib.load().mmf_enc_trunk_weight_bytes())
     return buf
 

@@ -556,15 +556,23 @@ def test_heads_backward_kernel_matches_autograd():
 
 
 # ---- image encoder trunk (SURVEY.md 8(f)-1): tcgen05 implicit-GEMM convolutions vs torch fp32 ---------------
-def _unmap(m, n, ch):
-    """bf16 hi/lo planes -> (n, ch, 32, 32) fp32"""
-    t = m.view(n, ops.enc_map_bytes(ch)).view(torch.bfloat16).reshape(n, ch // 8, 2, 1280, 8).float()
-    v = (t[:, :, 0] + t[:, :, 1])[:, :, 64:64 + 1088].reshape(n, ch // 8, 32, 34, 8)[:, :, :, :32]
-    return v.permute(0, 1, 4, 2, 3).reshape(n, ch, 32, 32)
+# A 32-channel activation map is [chunk of 8 channels 4][hi|lo][1280 positions][8 bf16]: a 64-position zero guard, then
+# position 34 y + x (two zero pad columns per row), then zeros.  mmf_enc_trunk's scratch holds four such maps per CTA.
+MAP32 = 4 * 2 * 1280 * 16  # 163,840 B
+
+
+def _unmap(maps):
+    """(m, MAP32) uint8 maps -> (m, 32, 32, 32) fp32 = hi + lo of every channel at every pixel"""
+    t = maps.view(torch.bfloat16).reshape(-1, 4, 2, 1280, 8).float()
+    v = (t[:, :, 0] + t[:, :, 1])[:, :, 64:64 + 1088].reshape(-1, 4, 32, 34, 8)[:, :, :, :32]
+    return v.permute(0, 1, 4, 2, 3).reshape(-1, 32, 32, 32)
 
 
 @pytest.mark.parametrize("n", [1, 37, 300])
-def test_encoder_conv_layers_match_torch(n):
+def test_encoder_trunk_layers_match_torch(n):
+    """Every layer of the fused trunk, read out of its own scratch: per CTA [x buf 0 | x buf 1 | t, later z | y].  CTA c
+    runs images c, c + G, ...; the k-th of them has its stem output in x[k & 1], so after the launch the maps hold
+    each CTA's last image (and, in the other x buffer, the previous one's stem output)."""
     import torch.nn.functional as F
     torch.manual_seed(n)
     img = (torch.rand(n, 32, 32, device=DEV) * 2 - 1).contiguous()
@@ -575,34 +583,39 @@ def test_encoder_conv_layers_match_torch(n):
     tol = 5e-5  # activations are kept as bf16 hi + lo (2^-18 relative); accumulation is fp32
     with torch.no_grad():
         x_ref = F.relu(c1(img[:, None]))
-        mx, mt, my = (ops.enc_new_map(n, 32, DEV) for _ in range(3))
-        mz = ops.enc_new_map(n, 16, DEV)
-        ops.enc_stem(img, ops.enc_pack_stem(c1), mx)
-        assert_close(_unmap(mx, n, 32).cpu(), x_ref.cpu(), tol, msg="5x5 stem")
-        ops.enc_conv3x3(n, 32, 32, mx, ops.enc_pack_conv3x3(c2a), relu=True, out_map=mt)
         t_ref = F.relu(c2a(x_ref))
-        assert_close(_unmap(mt, n, 32).cpu(), t_ref.cpu(), tol, msg="conv 32->32")
-        ops.enc_conv3x3(n, 32, 32, mt, ops.enc_pack_conv3x3(c2b), res_map=mx, relu=True, out_map=my)
         y_ref = F.relu(c2b(t_ref) + x_ref)
-        assert_close(_unmap(my, n, 32).cpu(), y_ref.cpu(), tol, msg="conv 32->32 + residual")
-        ops.enc_conv3x3(n, 32, 16, my, ops.enc_pack_conv3x3(c3), relu=True, out_map=mz)
         z_ref = F.relu(c3(y_ref))
-        assert_close(_unmap(mz, n, 16).cpu(), z_ref.cpu(), tol, msg="conv 32->16")
-        out = torch.empty(n, 8, 32, 32, device=DEV)
-        ops.enc_conv3x3(n, 16, 8, mz, ops.enc_pack_conv3x3(c4), relu=False, out_nchw=out)
-        assert_close(out.cpu(), c4(z_ref).cpu(), tol, msg="conv 16->8 (NCHW output)")
-        # the fused trunk (one launch, maps in L2-resident scratch) computes the same thing
+        out_ref = c4(z_ref)
         w = ops.enc_pack_trunk([c1, c2a, c2b, c3, c4])
         scratch = ops.enc_trunk_scratch(DEV)
-        fused_out = ops.enc_trunk(img, w, scratch, 8)
-        assert_close(fused_out.cpu(), c4(z_ref).cpu(), tol, msg="fused trunk")
-        assert torch.equal(fused_out, ops.enc_trunk(img, w, scratch, 8)), "fused trunk is not deterministic / scratch reuse"
-        # the zero guards and the pad columns of every map are still zero (the next layer's padding depends on it)
-        for m, ch in ((mx, 32), (mt, 32), (my, 32), (mz, 16)):
-            t = m.view(n, ch // 8, 2, 1280, 16)
-            assert int(t[:, :, :, :64].count_nonzero()) == 0 and int(t[:, :, :, 64 + 1088:].count_nonzero()) == 0
-            pads = t[:, :, :, 64:64 + 1088].reshape(n, ch // 8, 2, 32, 34, 16)[:, :, :, :, 32:]
-            assert int(pads.count_nonzero()) == 0
+        out = ops.enc_trunk(img, w, scratch, 8)
+        maps = scratch.cpu()
+    assert maps.numel() % (4 * MAP32) == 0
+    g_max = maps.numel() // (4 * MAP32)
+    G = min(g_max, n)
+    maps = maps.view(g_max, 4, MAP32)[:G]
+    ctas = torch.arange(G)
+    k_last = torch.tensor([len(range(c, n, G)) - 1 for c in range(G)])
+    last = ctas + G * k_last
+    x_last = _unmap(maps[ctas, k_last & 1])
+    tz = _unmap(maps[:, 2])
+    assert_close(x_last, x_ref[last].cpu(), tol, msg="layer 0: 5x5 stem + ReLU (x)")
+    assert_close(tz[:, 16:], t_ref[last, 16:].cpu(), tol, msg="layer 1: block1 32->32 + ReLU (t, channels 16-31)")
+    assert_close(_unmap(maps[:, 3]), y_ref[last].cpu(), tol, msg="layer 2: block2 32->32 + residual + ReLU (y)")
+    assert_close(tz[:, :16], z_ref[last].cpu(), tol, msg="layer 3: 32->16 + ReLU (z)")
+    # the previous image of a CTA left its stem output in the other x buffer (double-buffering parity)
+    prev = k_last >= 1
+    assert bool(prev.any()) == (n > G)
+    if n > G:
+        x_prev = _unmap(maps[ctas[prev], (k_last[prev] - 1) & 1])
+        assert_close(x_prev, x_ref[last[prev] - G].cpu(), tol, msg="layer 0 of the previous image (other x buffer)")
+    assert_close(out.cpu(), out_ref.cpu(), tol, msg="layer 4: 16->8 (NCHW output)")
+    assert torch.equal(out, ops.enc_trunk(img, w, scratch, 8)), "fused trunk is not deterministic / scratch reuse"
+    # the zero guards and the pad columns of every scratch map are still zero (the next layer's padding depends on it)
+    planes = maps.view(G, 4, 8, 1280, 16)
+    assert int(planes[..., :64, :].count_nonzero()) == 0 and int(planes[..., 64 + 1088:, :].count_nonzero()) == 0
+    assert int(planes[..., 64:64 + 1088, :].reshape(G, 4, 8, 32, 34, 16)[..., 32:, :].count_nonzero()) == 0
 
 
 @pytest.mark.parametrize("batch", [3, 16384 + 5])

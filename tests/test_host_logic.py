@@ -19,7 +19,7 @@ from oracle.make_golden import REFERENCE, reference_available
 from util import REPO, header_symbols, run_packed_chain, run_packed_rows
 
 
-def test_shared_library_exports_every_declared_symbol():
+def test_shared_library_matches_header_and_abi_version():
     assert os.path.exists(_lib.LIB_PATH), "run __graft_entry__.build() first"
     declared = header_symbols()
     assert len(declared) >= 16
@@ -30,7 +30,7 @@ def test_shared_library_exports_every_declared_symbol():
     assert not missing, missing
     lib = ctypes.CDLL(_lib.LIB_PATH)  # loads without a GPU; no compute call is made here
     lib.mmf_abi_version.restype = ctypes.c_int
-    assert lib.mmf_abi_version() == _lib.ABI_VERSION == 2
+    assert lib.mmf_abi_version() == _lib.ABI_VERSION == 3
 
 
 def test_library_contains_only_sm100a_code():
@@ -198,8 +198,8 @@ def _bf16_pairs(buf, count):
 
 @pytest.mark.parametrize("cin,cout", [(32, 32), (32, 16), (16, 8)])
 def test_conv3x3_operand_image_layout(cin, cout):
-    """mmf_enc_conv3x3's w_image: bf16 [tap 9][cin/8][2 npad rows: hi then lo][8] + fp32 bias[npad]; hi + lo restores
-    the fp32 weight to 2^-17 and padded rows are zero."""
+    """w_image of a 3x3 layer in mmf_enc_trunk's weights: bf16 [tap 9][cin/8][2 npad rows: hi then lo][8] + fp32
+    bias[npad]; hi + lo restores the fp32 weight to 2^-17 and padded rows are zero."""
     from multimodalfilter_b200 import ops
 
     torch.manual_seed(cin + cout)
@@ -215,21 +215,6 @@ def test_conv3x3_operand_image_layout(cin, cout):
     assert rebuilt[cout:].abs().max() == 0 if cout < npad else True
     bias = img[2 * n_w:].view(torch.float32)
     assert torch.equal(bias[:cout], conv.bias.detach()) and (bias[cout:] == 0).all()
-
-
-def test_conv3x3_dx_stacked_image_layout():
-    """MMF_ENC_VARIANT=3: bf16 [dy 3][cin/8][6 npad rows: hi dx-1 | hi dx0 | hi dx+1 | lo dx-1 | lo dx0 | lo dx+1][8]."""
-    from multimodalfilter_b200 import ops
-
-    torch.manual_seed(3)
-    conv = torch.nn.Conv2d(32, 16, 3, padding=1)
-    cin, cout, npad = 32, 16, 16
-    img = ops.enc_pack_conv3x3_dx(conv)
-    n_w = 3 * (cin // 8) * 6 * npad * 8
-    w = _bf16_pairs(img, n_w).reshape(3, cin // 8, 2, 3, npad, 8)       # (ky, chunk, hi|lo, kx, row, channel-in-chunk)
-    rebuilt = (w[:, :, 0] + w[:, :, 1]).permute(3, 1, 4, 0, 2).reshape(npad, cin, 3, 3)
-    ref = conv.weight.detach()
-    assert torch.allclose(rebuilt[:cout], ref, rtol=0, atol=float(ref.abs().max()) * 2 ** -16)
 
 
 def test_stem_and_trunk_weight_buffers():

@@ -11,5 +11,4 @@ timeout -k 10 600 python bench.py --impl reference --steps 2 --warmup 1 > gpurun
 timeout -k 10 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 80 --csv --log-file gpurun_out/launches.csv python tools/profile_step.py bf16x3 6 > gpurun_out/ncu_launch.log 2>&1
 timeout -k 10 900 ncu --set full --clock-control none --import-source on -k regex:k_particle_chain_tc -s 2 -c 1 -f -o gpurun_out/prof_chain_tc python tools/profile_step.py bf16x3 4 > gpurun_out/ncu_tc.log 2>&1; tail -1 gpurun_out/ncu_tc.log
 timeout -k 10 600 ncu --set full --clock-control none --import-source on -k regex:k_normalize_resample -s 2 -c 1 -f -o gpurun_out/prof_resample python tools/profile_step.py bf16x3 4 > gpurun_out/ncu_nr.log 2>&1; tail -1 gpurun_out/ncu_nr.log
-timeout -k 10 600 ncu --set full --clock-control none --import-source on -k regex:k_enc_trunk -s 2 -c 1 -f -o gpurun_out/prof_enc_trunk python tools/debug_enc.py 37 4096 300 > gpurun_out/ncu_enc.log 2>&1; tail -1 gpurun_out/ncu_enc.log
 ls -la gpurun_out | head -40
