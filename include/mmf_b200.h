@@ -248,6 +248,33 @@ int mmf_ekf_loop_bwd(const mmf_ekf_model* models, int32_t num_filters, int32_t T
 int mmf_dynamics_jacobian(const mmf_ekf_model* model, int32_t N, const float* states,
                           const float* controls, float* pred_out, float* jac_out, void* stream);
 
+/* ---- dynamics training: open-loop rollout with a tape, and its reverse mode ---------------------------------------
+ * DynamicsModel.forward_loop (A.4; ref: crossmodal/eval_helpers.py:135-137) of the gated-residual dynamics `chain`
+ * (in_dim = sd, out_dim = sd + 1), T steps in ONE launch, a warp per trajectory:
+ *   h = chain(x_t, rowbias[t]);   x_{t+1} = x_t + h[:sd] * sigmoid(h[sd]);   states_out[t] = x_{t+1}   (x_0 = x0)
+ * x0 (N,sd), states_out (T,N,sd).  rowbias (T,N,64) = the hoisted control rows (mmf_chain's `rowbias`) given by the
+ * caller, or NULL: then `rows` (with the control encoder) and controls (T,N,cd) compute them inside the kernel.
+ * act_out (L+1, 16, T*N, 4), NULL = no tape, L = 2 n_pre_res + 1 + 2 n_post_res: chunk-major planes in the layout of
+ * mmf_pf_heads_weight_grads (element [l][c][p][j] = column 4c+j of row p, rows p = t*N + n): plane l = the input of
+ * 64x64 layer l, plane L = the input of the output layer.  The arithmetic is the same with and without the tape, so
+ * states_out is bit-identical either way. */
+int mmf_dyn_rollout_fwd(const mmf_chain* chain, const mmf_traj_rows* rows, int32_t T, int32_t N, const float* x0,
+                        const float* controls, const float* rowbias, float* states_out, float* act_out, void* stream);
+
+/* Reverse mode of mmf_dyn_rollout_fwd from its tape, one warp per trajectory walking t = T-1 ... 0.  With xb the gradient
+ * reaching states[t] (d_states[t] plus what step t+1 sent back), y = the output layer recomputed from plane L,
+ * g = sigmoid(y[sd]):
+ *   d_y[t]  = yb:   yb_i = xb_i g (i < sd),   yb_sd = g (1 - g) sum_i xb_i y_i
+ *   delta through W_out, the resblocks, the mid layer and the input layer, each ReLU mask read from the tape (the output
+ *   of layer l is plane l+1, that of the input layer plane 0; the mid layer is masked only when mid_relu);
+ *   d rowbias[t] = delta of the mid layer (plane 2 n_pre_res);   xb(t-1) = xb + in_W^T delta_in;   d_x0 = xb(-1).
+ * d_states (T,N,sd) may be NULL (= zero).  delta_out (L+1, 16, T*N, 4) in the tape's layout: plane l = delta of 64x64
+ * layer l, plane L = delta of the input layer (the convention of mmf_pf_heads_backward, so mmf_pf_heads_weight_grads with
+ * K = 1 and x = the step inputs (x0, states[0 .. T-2]) reduces the parameter gradients); d_y_out (T*N, sd+1) = delta of
+ * the output layer; d_x0_out (N,sd).  Every element is written by one lane, no atomics: bit-reproducible. */
+int mmf_dyn_rollout_bwd(const mmf_chain* chain, int32_t T, int32_t N, const float* act, const float* d_states,
+                        float* delta_out, float* d_y_out, float* d_x0_out, void* stream);
+
 /* R10  CrossmodalKalmanFilter.calculate_weighted_states (ref: base_models/crossmodal_kf.py:153-167,
  * utility.py:4-11): rows = T*N independent fusions.
  *   mean = sum_k (beta_k / (sum_k beta_k + 1e-9)) * mu_k ;  cov = sum_k (beta_k beta_k^T) o P_k

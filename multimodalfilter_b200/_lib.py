@@ -117,6 +117,8 @@ PROTOTYPES = {
         C.c_int,
         [C.POINTER(EKFModel), _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     ),
+    "mmf_dyn_rollout_fwd": (C.c_int, [C.POINTER(Chain), C.POINTER(TrajRows), _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mmf_dyn_rollout_bwd": (C.c_int, [C.POINTER(Chain), _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mmf_dynamics_jacobian": (C.c_int, [C.POINTER(EKFModel), _i32, _vp, _vp, _vp, _vp, _vp]),
     "mmf_kf_fuse_crossmodal": (C.c_int, [_i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mmf_pf_forward_loop_persistent": (C.c_int, [_i32, _i32]),

@@ -321,6 +321,53 @@ int mmf_dynamics_jacobian(const mmf_ekf_model* model, int32_t N, const float* st
   return launch_ekf(P, model->state_dim, (cudaStream_t)stream);
 }
 
+static int validate_dyn_chain(const mmf_chain* chain, const char* what) {
+  MMF_REQUIRE(chain != nullptr, "%s: chain is NULL", what);
+  MMF_REQUIRE(chain->in_dim >= 1 && chain->in_dim <= MMF_MAX_SD, "%s: state_dim %d outside 1..%d", what, chain->in_dim,
+              MMF_MAX_SD);
+  return validate_chain(*chain, chain->in_dim, chain->in_dim + 1, what);
+}
+
+int mmf_dyn_rollout_fwd(const mmf_chain* chain, const mmf_traj_rows* rows, int32_t T, int32_t N, const float* x0,
+                        const float* controls, const float* rowbias, float* states_out, float* act_out, void* stream) {
+  int rc = validate_dyn_chain(chain, "dyn_rollout");
+  if (rc) return rc;
+  MMF_REQUIRE(T >= 0 && N >= 0, "dyn_rollout: bad shape T=%d N=%d", T, N);
+  MMF_REQUIRE((long long)T * N <= 0x7fffffffLL, "dyn_rollout: T * N = %lld rows", (long long)T * N);
+  if (T == 0 || N == 0) return MMF_OK;
+  MMF_REQUIRE(x0 && states_out, "dyn_rollout: NULL buffer");
+  DynRolloutParams P;
+  memset(&P, 0, sizeof(P));
+  P.ch = to_dev(*chain);
+  if (rowbias == nullptr) {
+    MMF_REQUIRE(rows && controls && rows->w && rows->has_encoder && rows->in_dim >= 1 && rows->in_dim <= MMF_MAX_CD,
+                "dyn_rollout: without rowbias the control rows (with encoder, 1..%d inputs) and the controls are needed",
+                MMF_MAX_CD);
+    P.rows = to_dev(*rows);
+    P.cd = rows->in_dim;
+  }
+  P.T = T; P.N = N;
+  P.x0 = x0; P.controls = controls; P.rowbias = rowbias; P.states_out = states_out; P.act_out = act_out;
+  return launch_dyn_rollout(P, (cudaStream_t)stream);
+}
+
+int mmf_dyn_rollout_bwd(const mmf_chain* chain, int32_t T, int32_t N, const float* act, const float* d_states,
+                        float* delta_out, float* d_y_out, float* d_x0_out, void* stream) {
+  int rc = validate_dyn_chain(chain, "dyn_rollout_bwd");
+  if (rc) return rc;
+  MMF_REQUIRE(T >= 0 && N >= 0, "dyn_rollout_bwd: bad shape T=%d N=%d", T, N);
+  MMF_REQUIRE((long long)T * N <= 0x7fffffffLL, "dyn_rollout_bwd: T * N = %lld rows", (long long)T * N);
+  if (N == 0) return MMF_OK;
+  MMF_REQUIRE(d_x0_out, "dyn_rollout_bwd: NULL buffer");
+  MMF_REQUIRE(T == 0 || (act && delta_out && d_y_out), "dyn_rollout_bwd: NULL buffer");
+  DynRolloutBwdParams P;
+  memset(&P, 0, sizeof(P));
+  P.ch = to_dev(*chain);
+  P.T = T; P.N = N;
+  P.act = act; P.d_states = d_states; P.delta_out = delta_out; P.d_y_out = d_y_out; P.d_x0_out = d_x0_out;
+  return launch_dyn_rollout_bwd(P, (cudaStream_t)stream);
+}
+
 int mmf_kf_fuse_crossmodal(int32_t K, int32_t rows, int32_t sd, const float* mu, const float* P, const float* beta,
                            float* mean_out, float* cov_out, void* stream) {
   MMF_REQUIRE(K >= 1 && rows >= 0 && sd >= 1 && sd <= MMF_MAX_SD, "kf_fuse: bad shape K=%d rows=%d sd=%d", K, rows, sd);

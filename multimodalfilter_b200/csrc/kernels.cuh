@@ -58,6 +58,33 @@ struct EkfBwdParams {
   float* d_r_tril;        // (F, T, N, sd, sd)
 };
 
+// Open-loop rollout of the gated-residual dynamics (k_dyn_rollout) and its reverse mode (k_dyn_rollout_bwd).
+struct DynRolloutParams {
+  ChainDev ch;
+  TrajRowsDev rows;
+  int T, N, cd;
+  const float* x0;        // (N, sd)
+  const float* controls;  // (T, N, cd)   read when rowbias == NULL (rows computed in the kernel)
+  const float* rowbias;   // (T, N, 64)   or NULL
+  float* states_out;      // (T, N, sd)
+  float* act_out;         // (L+1, 16, T*N, 4) tape, or NULL
+};
+
+struct DynRolloutBwdParams {
+  ChainDev ch;
+  int T, N;
+  const float* x0;        // (N, sd)
+  const float* states;    // (T, N, sd)
+  const float* act;       // (L+1, 16, T*N, 4)
+  const float* d_states;  // (T, N, sd) or NULL
+  float* delta_out;       // (L+1, 16, T*N, 4)
+  float* d_y_out;         // (T*N, sd+1)
+  float* d_x0_out;        // (N, sd)
+};
+
+int launch_dyn_rollout(const DynRolloutParams& P, cudaStream_t stream);
+int launch_dyn_rollout_bwd(const DynRolloutBwdParams& P, cudaStream_t stream);
+
 int launch_particle_chain_ffma(const mmf_pf_model* model, int N, int M, const float* states_in, const float* eps,
                                const float* rowbias, const float* logw_in, const float* modw, uint32_t enabled,
                                float* states_out, float* logw_out, float* ll_out, cudaStream_t stream,

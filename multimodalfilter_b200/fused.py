@@ -145,6 +145,7 @@ class _DynamicsSpec:
             return
         self.dyn, self.sd, self.cd = dyn, sd, ct[0].in_features
         self.state, self.control, self.shared = st, ct, sh
+        self.feat_dim = U  # the state columns of the mid Linear start after the control features
         self.ok = 1 <= sd <= _lib.MAX_SD and 1 <= self.cd <= _lib.MAX_CD
 
     def pack(self):
@@ -395,6 +396,18 @@ class EKFPlan:
         """``loop`` plus the tape of the backward: -> means, covs, pred (F,T,N,sd), jac (F,T,N,sd,sd)."""
         self.refresh(z.device)
         return ops.ekf_loop_train(self.structs, mean0, cov0, controls, z, r_tril)
+
+    def rollout(self, x0, controls=None, rowbias=None):
+        """Open-loop rollout of the first filter's dynamics (``DynamicsModel.forward_loop``) in one launch: x0 (N,sd) and
+        controls (T,N,cd) or the hoisted rows (T,N,64) -> states (T,N,sd)."""
+        self.refresh(x0.device)
+        m = self.structs[0]
+        return ops.dyn_rollout(m.dynamics, m.dynamics_rows, x0, controls, rowbias)
+
+    def rollout_train(self, x0, rowbias):
+        """``rollout`` from given rows that also records the tape: -> states (T,N,sd), act (L+1,16,T*N,4)."""
+        self.refresh(x0.device)
+        return ops.dyn_rollout_train(self.structs[0].dynamics, x0, rowbias)
 
     def jacobian(self, which, states, controls):
         self.refresh(states.device)

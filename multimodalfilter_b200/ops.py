@@ -494,6 +494,65 @@ def ekf_loop_bwd(model_structs, cov0, z, r_tril, covs, pred, jac, d_means=None, 
     return d_mean0, d_cov0, d_z, d_r
 
 
+def dyn_depth(chain):
+    return 2 * chain.n_pre_res + 1 + 2 * chain.n_post_res
+
+
+def dyn_rollout(chain, rows, x0, controls=None, rowbias=None):
+    """Open-loop rollout of the dynamics chain, T steps in one launch: x0 (N,sd) and either controls (T,N,cd) (the control
+    rows are computed inside the kernel from ``rows``) or rowbias (T,N,64) -> states (T,N,sd)."""
+    lib = _lib.load()
+    x0 = _f32c(x0)
+    N, sd = x0.shape
+    src = rowbias if rowbias is not None else controls
+    T = src.shape[0]
+    assert src.shape[1] == N and (rowbias is None or rowbias.shape == (T, N, _lib.UNITS)), tuple(src.shape)
+    src = _f32c(src)
+    states = torch.empty((T, N, sd), device=x0.device, dtype=torch.float32)
+    _lib.check(
+        PROFILE.run("dyn_rollout", 1, lib.mmf_dyn_rollout_fwd, C.byref(chain), C.byref(rows), T, N, _lib.ptr(x0),
+                    None if rowbias is not None else _lib.ptr(src), _lib.ptr(src) if rowbias is not None else None,
+                    _lib.ptr(states), None, _lib.stream_of(x0))
+    )
+    return states
+
+
+def dyn_rollout_train(chain, x0, rowbias):
+    """``dyn_rollout`` with the given rows that also records the tape of ``dyn_rollout_bwd``: x0 (N,sd), rowbias (T,N,64)
+    -> states (T,N,sd), act (L+1,16,T*N,4): plane l = input of 64x64 layer l, plane L = input of the output layer."""
+    lib = _lib.load()
+    x0, rowbias = _f32c(x0), _f32c(rowbias)
+    N, sd = x0.shape
+    T = rowbias.shape[0]
+    assert rowbias.shape == (T, N, _lib.UNITS), tuple(rowbias.shape)
+    states = torch.empty((T, N, sd), device=x0.device, dtype=torch.float32)
+    act = torch.empty((dyn_depth(chain) + 1, _lib.UNITS // 4, T * N, 4), device=x0.device, dtype=torch.float32)
+    _lib.check(
+        PROFILE.run("dyn_rollout_train", 1, lib.mmf_dyn_rollout_fwd, C.byref(chain), None, T, N, _lib.ptr(x0), None,
+                    _lib.ptr(rowbias), _lib.ptr(states), _lib.ptr(act), _lib.stream_of(x0))
+    )
+    return states, act
+
+
+def dyn_rollout_bwd(chain, T, N, act, d_states=None):
+    """Reverse mode of ``dyn_rollout_train`` from its tape: d_states (T,N,sd) | None -> delta (L+1,16,T*N,4) (plane l =
+    delta of 64x64 layer l, plane L = delta of the input layer), d_y (T*N, sd+1) (delta of the output layer), d_x0 (N,sd)."""
+    lib = _lib.load()
+    sd = chain.in_dim
+    act = _f32c(act)
+    assert act.shape == (dyn_depth(chain) + 1, _lib.UNITS // 4, T * N, 4), tuple(act.shape)
+    d_states = None if d_states is None else _f32c(d_states)
+    assert d_states is None or d_states.shape == (T, N, sd)
+    delta = torch.empty_like(act)
+    d_y = torch.empty((T * N, sd + 1), device=act.device, dtype=torch.float32)
+    d_x0 = torch.empty((N, sd), device=act.device, dtype=torch.float32)
+    _lib.check(
+        PROFILE.run("dyn_rollout_bwd", 1, lib.mmf_dyn_rollout_bwd, C.byref(chain), T, N, _lib.ptr(act), _lib.ptr(d_states),
+                    _lib.ptr(delta), _lib.ptr(d_y), _lib.ptr(d_x0), _lib.stream_of(act))
+    )
+    return delta, d_y, d_x0
+
+
 def dynamics_jacobian(model_struct, states, controls):
     """A.4: states (N,sd), controls (N,cd) -> pred (N,sd), jacobian (N,sd,sd)."""
     lib = _lib.load()

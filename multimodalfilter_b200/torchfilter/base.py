@@ -62,10 +62,18 @@ class DynamicsModel(nn.Module, abc.ABC):
         """-> (predicted states (N, sd), scale_tril (N, sd, sd))"""
 
     def forward_loop(self, *, initial_states, controls):
-        """Open-loop rollout (used at ref: crossmodal/eval_helpers.py:135-137)."""
+        """Open-loop rollout (used at ref: crossmodal/eval_helpers.py:135-137).  Recognised gated-residual dynamics with
+        CUDA fp32 inputs run the T steps in one kernel launch (and, when a gradient is needed, the reverse mode in one
+        more: ``training.dynamics_rollout``); anything else runs the modules step by step."""
         ctrl = SliceWrapper(controls)
         T, N = ctrl.shape[:2]
         assert initial_states.shape == (N, self.state_dim)
+        from .. import training
+
+        states = training.dynamics_rollout(self, initial_states, controls)
+        if states is not None:
+            q = self.Q_scale_tril if hasattr(self, "Q_scale_tril") else torch.diag(self.Q_scale_tril_diag)
+            return states, q.expand(T, N, self.state_dim, self.state_dim).contiguous()
         states, trils, x = [], [], initial_states
         for t in range(T):
             x, tril = self(initial_states=x, controls=ctrl[t])

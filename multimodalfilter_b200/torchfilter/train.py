@@ -8,6 +8,7 @@ the optimiser step is ``buddy.minimize``, which all-reduces the gradients first 
 import torch
 import torch.nn.functional as F
 
+from .. import training
 from ..fannypack import utils as fp_utils
 from ..fannypack.utils import SliceWrapper
 from . import base
@@ -64,7 +65,10 @@ def train_dynamics_single_step(buddy, dynamics_model, dataloader, *, loss_functi
     with buddy.log_scope(optimizer_name):
         for batch in dataloader:
             prev, nxt, _observations, controls = fp_utils.to_device(batch, buddy.device)
-            pred, _ = dynamics_model(initial_states=prev, controls=controls)
+            # recognised dynamics on CUDA: one step of the fused rollout (T = 1) and its reverse mode
+            fused = training.dynamics_rollout(dynamics_model, prev, controls[None]) \
+                if isinstance(controls, torch.Tensor) else None
+            pred = fused[0] if fused is not None else dynamics_model(initial_states=prev, controls=controls)[0]
             loss = loss_fn(pred, nxt)
             buddy.minimize(loss, optimizer_name=optimizer_name)
             total += float(loss.detach())

@@ -14,12 +14,18 @@ wrapped in one ``torch.autograd.Function``; the fusion log-sum-exp, the normalis
 estimate are (N, M)-sized torch ops that autograd differentiates itself, and the per-trajectory
 pieces (observation encoders, the observation half of the first shared Linear, the modality weight
 model) stay ordinary torch modules, so their gradients come from autograd as well.
+
+``FusedDynamicsRollout`` trains the dynamics themselves (the pre-training phases ``train_dynamics_single_step`` /
+``train_dynamics_recurrent``): the open-loop rollout of T steps is one launch that records every layer's input, and its
+reverse mode one more; the control branch and the control half of the mid Linear stay torch ops over all T*N rows.
 """
+import types
 from typing import List
 
 import torch
+import torch.nn.functional as F
 
-from . import _lib, ops
+from . import _lib, fused, ops
 
 U = _lib.UNITS
 
@@ -244,3 +250,86 @@ def fused_train_applicable(filt, plan, resample: bool) -> bool:
     if filt.particle_states.requires_grad:
         return False
     return not any(p.requires_grad for p in filt.dynamics_model.parameters())
+
+
+class FusedDynamicsRollout(torch.autograd.Function):
+    """(plan, x0 (N,sd), rowbias (T,N,64), the state-chain parameters in ``head_parameters`` order) -> states (T,N,sd):
+    the open-loop rollout of the plan's dynamics in one launch that records the tape (``mmf_dyn_rollout_fwd``), and its
+    reverse mode in one more (``mmf_dyn_rollout_bwd``).  The backward returns d x0, d rowbias (the mid layer's delta) and
+    the parameter gradients, reduced by ``mmf_pf_heads_weight_grads`` (K = 1) from the tape and the deltas; the
+    (sd+1)-wide output layer's gradients are one matmul and one sum over d_y.  Only the state half of the mid Linear's
+    weight is set: its control half and its bias receive their gradient through rowbias."""
+
+    @staticmethod
+    def forward(ctx, plan, x0, rowbias, *params):
+        x0 = x0.detach().contiguous()
+        states, act = plan.rollout_train(x0, rowbias.detach().contiguous())
+        # the struct and the weight buffers it points at, as of this forward
+        ctx.spec, ctx.chain, ctx.buffers = plan.dyns[0], plan.structs[0].dynamics, plan._buffers
+        ctx.save_for_backward(x0, states, act)
+        return states
+
+    @staticmethod
+    def backward(ctx, d_states):
+        x0, states, act = ctx.saved_tensors
+        T, N, sd = states.shape
+        spec = ctx.spec
+        delta, d_y, d_x0 = ops.dyn_rollout_bwd(ctx.chain, T, N, act, d_states)
+        d_rows = delta[mid_layer_index(spec)].view(U // 4, T, N, 4).permute(1, 2, 0, 3).reshape(T, N, U)
+        need = ctx.needs_input_grad[3:]
+        grads = [None] * len(need)
+        if any(need):
+            x_in = torch.cat([x0[None], states[:-1]]).reshape(T * N, sd)  # the input of every step, rows (t, n)
+            no_head = d_y.new_zeros((1, T * N))  # the kernel's 1-wide output layer is not this chain's
+            dW, db, g_in, g_out = ops.pf_heads_weight_grads(act[None], delta[None], x_in, no_head)
+            grads, _ = _grads_for_head(spec, dW[0], db[0], g_in[0], g_out[0], d_y.new_zeros(1))
+            grads[-2:] = [d_y.t() @ ops.rows_view(act[-1]), d_y.sum(dim=0)]  # the (sd+1)-wide output layer
+            grads = [g if n else None for g, n in zip(grads, need)]
+        return (None, d_x0 if ctx.needs_input_grad[1] else None, d_rows if ctx.needs_input_grad[2] else None, *grads)
+
+
+def _dynamics_plan(dyn):
+    """The packed-weight plan of a dynamics model (shared with ``DynamicsModel.jacobian``), or False if unrecognised."""
+    plan = dyn.__dict__.get("_mmf_jac_plan")
+    if plan is None:
+        plan = fused.EKFPlan.build([types.SimpleNamespace(dynamics_model=dyn)]) or False
+        dyn.__dict__["_mmf_jac_plan"] = plan
+    return plan
+
+
+def dynamics_structure_ok(dyn, controls) -> bool:
+    """The checks of ``dynamics_rollout`` that need no device: ``dyn.fused_train`` (default on), controls a (T, N, cd)
+    tensor with T >= 1 (not a dict), no forward or pre-forward hook on the dynamics or its submodules (the fused path
+    never calls the modules of the state chain), and dynamics recognised by ``fused._DynamicsSpec``."""
+    if not getattr(dyn, "fused_train", True):
+        return False
+    if not isinstance(controls, torch.Tensor) or controls.dim() != 3 or controls.shape[0] < 1:
+        return False
+    if any(m._forward_hooks or m._forward_pre_hooks for m in dyn.modules()):
+        return False
+    return bool(_dynamics_plan(dyn))
+
+
+def dynamics_rollout(dyn, x0, controls):
+    """Open-loop rollout of ``dyn`` from x0 (N, sd) under controls (T, N, cd) through the rollout kernels -> states
+    (T, N, sd), or None when they do not apply (``dynamics_structure_ok`` fails, or x0 / controls are not CUDA fp32 tensors
+    of matching shape): the caller then runs its generic loop.  When a gradient is needed (grad mode on and a dynamics
+    parameter, x0 or the controls requires it) the rows go through torch autograd and the chain through
+    ``FusedDynamicsRollout``; otherwise the rows are computed inside the single rollout launch."""
+    tensors = (x0, controls)
+    if not all(isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float32 for t in tensors):
+        return None
+    if not dynamics_structure_ok(dyn, controls):
+        return None
+    plan = _dynamics_plan(dyn)
+    T, N, cd = controls.shape
+    if x0.shape != (N, plan.sd) or cd != plan.cd:
+        return None
+    spec = plan.dyns[0]
+    params = head_parameters(spec)
+    if torch.is_grad_enabled() and (x0.requires_grad or controls.requires_grad or
+                                    any(p.requires_grad for p in dyn.parameters())):
+        mid = spec.shared[0]
+        rows = F.linear(spec.dyn.control_layers(controls.reshape(T * N, cd)), mid.weight[:, :U], mid.bias)
+        return FusedDynamicsRollout.apply(plan, x0, rows.reshape(T, N, U), *params)
+    return plan.rollout(x0, controls)
