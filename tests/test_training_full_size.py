@@ -40,11 +40,12 @@ from multimodalfilter_b200 import _lib, fused, ops  # noqa: E402
 from multimodalfilter_b200.crossmodal import models as M  # noqa: E402
 from multimodalfilter_b200.synthetic import fill_parameters, synthetic_trajectories  # noqa: E402
 
-from util import ReplayNoise, draw_noise, kernel_ran  # noqa: E402
+from full_size import (  # noqa: E402
+    GROUPS, TILE, assert_rows, chain_layers, chain_regime, dynamics_moved, nm_for_tiles, profiled)
+from util import ReplayNoise, draw_noise  # noqa: E402
 
 DEV = "cuda:0"
 U = _lib.UNITS
-TILE, GROUPS = 128, 4        # chain kernels: rows per tile, groups (tiles in flight) per CTA
 DWT_ROWS = 64                # k_heads_dw_tc: rows per tile
 C4_N, C4_M = 8192, 30
 FWD = "k_particle_chain_ws<4,2,true>"
@@ -70,17 +71,6 @@ def _sms():
 
 
 # ---- the launchers' arithmetic, restated ----------------------------------------------------------------------------
-def chain_regime(P, sms):
-    """k_particle_chain_ws / k_head_chain_bwd: ceil(tiles / 4) CTAs of 4 groups, at most one per SM; slot s covers tiles
-    4 s .. 4 s + 3 and CTA u takes slots u, u + CTAs, ...  Returns the tiles of the busiest group, the tiles of the last
-    slot (the issuer's `ng`), the rows of the last tile and the CTA count."""
-    tiles = -(-P // TILE)
-    slots = -(-tiles // GROUPS)
-    ctas = min(slots, sms)
-    return {"tiles": tiles, "ctas": ctas, "tiles_per_group": -(-slots // ctas),
-            "last_slot": tiles - GROUPS * (slots - 1), "last_tile_rows": P - TILE * (tiles - 1)}
-
-
 def dw_partition(K, L, P, sms):
     """particle_chain_bwd.cu dw_partition: (dw_chunks, dw_rows, edge_chunks, edge_rows)."""
     chunks = (sms * 3 + K * L - 1) // (K * L)
@@ -99,13 +89,6 @@ def dw_regime(K, L, P, sms):
     last = P - rows * (chunks - 1)
     return {"chunks": chunks, "tiles_per_chunk": rows // DWT_ROWS, "last_chunk_rows": last,
             "last_chunk_tiles": -(-last // DWT_ROWS), "ragged": last % DWT_ROWS != 0}
-
-
-def nm_for_tiles(tiles, M):
-    """(N, M) with N M inside the last tile of `tiles` tiles and not a multiple of 128 (a ragged last tile)."""
-    N = (tiles * TILE - 1) // M
-    assert (tiles - 1) * TILE < N * M < tiles * TILE
-    return N, M
 
 
 def chain_shapes(sms):
@@ -127,73 +110,6 @@ def assert_chain_regime(case, P, sms):
         assert g["tiles"] == GROUPS * sms * k + r and g["ctas"] == sms, g
         assert g["tiles_per_group"] == k + 1 and g["last_slot"] == r and 0 < g["last_tile_rows"] < TILE, g
     return g
-
-
-def profiled(fn, wants):
-    from torch.profiler import ProfilerActivity, profile
-
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        out = fn()
-        torch.cuda.synchronize()
-    names = {e.name for e in prof.events()}
-    for w in wants:
-        assert kernel_ran(names, w), f"{w} did not run; kernels: {sorted(names)}"
-    return out
-
-
-# ---- float64 chains -------------------------------------------------------------------------------------------------
-def _d(t):
-    return t.detach().double()
-
-
-def chain_layers(state, shared, feat_cols):
-    """The 64x64 layers of a chain as (W (64, 64), b or None, kind) with kind RES_A / RES_B / MID, then the input and
-    the output Linear.  feat_cols: the mid layer's state columns."""
-    (in_lin, pre), (mid, post, out) = state, shared
-    layers = []
-    for r in pre:
-        layers += [(_d(r.block1.weight), _d(r.block1.bias), "A"), (_d(r.block2.weight), _d(r.block2.bias), "B")]
-    layers.append((_d(mid.weight[:, feat_cols]), None, "MID"))
-    for r in post:
-        layers += [(_d(r.block1.weight), _d(r.block1.bias), "A"), (_d(r.block2.weight), _d(r.block2.bias), "B")]
-    return (_d(in_lin.weight), _d(in_lin.bias)), layers, (_d(out.weight), _d(out.bias))
-
-
-def dynamics_moved(plan, states, eps, rowbias0, Mp):
-    """x' = x + h[:sd] sigmoid(h[sd]) + q_tril eps through the float64 dynamics chain (mid layer linear)."""
-    sd = plan.sd
-    (Wi, bi), layers, (Wo, bo) = chain_layers(plan.dyn.state, plan.dyn.shared, slice(U, 2 * U))
-    x = states.reshape(-1, sd).double()
-    rb = rowbias0.double().repeat_interleave(Mp, dim=0)
-    h = torch.relu(x @ Wi.T + bi)
-    res = None
-    for W, b, kind in layers:
-        if kind == "MID":
-            h = h @ W.T + rb
-        elif kind == "A":
-            res, h = h, torch.relu(h @ W.T + b)
-        else:
-            h = torch.relu(h @ W.T + b + res)
-    y = h @ Wo.T + bo
-    q = plan.dyn.q()[: sd * sd].reshape(sd, sd).double().to(x.device)
-    return x + y[:, :sd] * torch.sigmoid(y[:, sd:sd + 1]) + eps.double() @ q.T
-
-
-def row_excess(got, ref, bar):
-    """Worst |got - ref| / max(|ref|, rms(ref)) over the entries of each row, in units of `bar`: (worst, its row).  A NaN
-    in `got` counts as infinitely wrong."""
-    got, ref = got.reshape(got.shape[0], -1).double(), ref.reshape(ref.shape[0], -1).double()
-    scale = ref.pow(2).mean().sqrt()
-    err = (got - ref).abs() / torch.maximum(ref.abs(), scale)
-    per_row = torch.nan_to_num(err, nan=math.inf).amax(dim=1) / bar
-    worst, row = per_row.max(dim=0)
-    return float(worst), int(row)
-
-
-def assert_rows(got, ref, bar, what, report, category):
-    worst, row = row_excess(got, ref, bar)
-    report[category] = max(report.get(category, 0.0), worst * bar)
-    assert worst <= 1.0, f"{what}: {worst:.2f}x the bar {bar:g} at row {row} (tile {row // TILE})"
 
 
 # ---- raw entry points with NaN-prefilled outputs -------------------------------------------------------------------
