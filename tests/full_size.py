@@ -1,5 +1,6 @@
-"""Helpers of the full-size kernel tests (test_training_full_size.py, test_inference_full_size.py): the chain launchers'
-tile arithmetic restated, float64 evaluations of the packed chains, and per-row error reports."""
+"""Helpers of the full-size kernel tests (test_training_full_size.py, test_inference_full_size.py,
+test_kalman_full_size.py): the chain launchers' tile arithmetic restated, float64 evaluations of the packed chains, and
+per-row error reports."""
 import math
 
 import torch
@@ -59,20 +60,31 @@ def chain_layers(state, shared, feat_cols):
     return (_d(in_lin.weight), _d(in_lin.bias)), layers, (_d(out.weight), _d(out.bias))
 
 
-def chain_forward(state, shared, feat_cols, x, rb, mid_relu):
-    """A whole chain in float64 on rows x (P, in_dim) with the hoisted mid-layer rows rb (P, 64): (P, out_dim)."""
+def chain_forward(state, shared, feat_cols, x, rb, mid_relu, planes=None, preacts=None):
+    """A whole chain in float64 on rows x (P, in_dim) with the hoisted mid-layer rows rb (P, 64): (P, out_dim).
+    `planes`, a list, receives the input of every 64x64 layer and then that of the output layer (a tape's planes);
+    `preacts`, a list, the input of every ReLU."""
+    def relu(a):
+        if preacts is not None:
+            preacts.append(a)
+        return torch.relu(a)
+
     (Wi, bi), layers, (Wo, bo) = chain_layers(state, shared, feat_cols)
-    h = torch.relu(x @ Wi.T + bi)
+    h = relu(x @ Wi.T + bi)
     res = None
     for W, b, kind in layers:
+        if planes is not None:
+            planes.append(h)
         if kind == "MID":
             h = h @ W.T + rb
             if mid_relu:
-                h = torch.relu(h)
+                h = relu(h)
         elif kind == "A":
-            res, h = h, torch.relu(h @ W.T + b)
+            res, h = h, relu(h @ W.T + b)
         else:
-            h = torch.relu(h @ W.T + b + res)
+            h = relu(h @ W.T + b + res)
+    if planes is not None:
+        planes.append(h)
     return h @ Wo.T + bo
 
 
@@ -93,8 +105,8 @@ def head_ll(spec, x, rb):
 
 # ---- per-row errors -------------------------------------------------------------------------------------------------
 def row_excess(got, ref, bar):
-    """Worst |got - ref| / max(|ref|, rms(ref)) over the entries of each row, in units of `bar`: (worst, its row).  A NaN
-    in `got` counts as infinitely wrong."""
+    """Worst |got - ref| / max(|ref|, rms(ref)) over the entries of each row, in units of `bar` (a number, or a tensor of
+    one bar per row): (worst, its row).  A NaN in `got` counts as infinitely wrong."""
     got, ref = got.reshape(got.shape[0], -1).double(), ref.reshape(ref.shape[0], -1).double()
     scale = ref.pow(2).mean().sqrt()
     err = (got - ref).abs() / torch.maximum(ref.abs(), scale)
@@ -103,7 +115,11 @@ def row_excess(got, ref, bar):
     return float(worst), int(row)
 
 
-def assert_rows(got, ref, bar, what, report, category):
+def assert_rows(got, ref, bar, what, report, category, where=None):
+    """row_excess within the bar; `report[category]` keeps the worst relative error.  `where(row)` names a failing row
+    (default: its 128-row tile)."""
     worst, row = row_excess(got, ref, bar)
-    report[category] = max(report.get(category, 0.0), worst * bar)
-    assert worst <= 1.0, f"{what}: {worst:.2f}x the bar {bar:g} at row {row} (tile {row // TILE})"
+    bar_at = float(bar[row]) if torch.is_tensor(bar) else bar
+    report[category] = max(report.get(category, 0.0), worst * bar_at)
+    label = where(row) if where is not None else f"tile {row // TILE}"
+    assert worst <= 1.0, f"{what}: {worst:.2f}x the bar {bar_at:g} at row {row} ({label})"
