@@ -396,6 +396,55 @@ int mmf_row_mlp(int64_t rows, const mmf_mlp_op* ops, int32_t n_ops, const float*
                 const int32_t* out_dims, const int32_t* out_slots, int32_t n_outputs, int32_t scratch_floats,
                 void* stream);
 
+/* Training of an mmf_row_mlp program (reverse mode of the ops above).  Rows are taken in groups of 8 (G = ceil(rows/8)
+ * groups, the last one padded); per-row planes are stored group-major and feature-major inside a group:
+ *     element (row, f) of a plane with F floats per row is at  [(row / 8) * F + f] * 8 + row % 8
+ * so the 8 rows a warp owns are 32 contiguous bytes per feature.
+ *   tape    F_tape = sum over ops of (in_dim + out_dim) floats per row, G * 8 * F_tape floats in all: op o's input
+ *           (src) at f = T_o, its post-activation output (dst) at f = T_o + in_dim, T_o = sum_{p<o} (in_dim + out_dim).
+ *   delta   F_delta = sum over ops of out_dim, G * 8 * F_delta floats: g_o = d loss / d (pre-activation of op o)
+ *           at f = sum_{p<o} out_dim.  Rows past the end of the padded last group hold zeros.
+ * mmf_row_mlp_train_sizes: the float counts of both planes and the byte size of the weight-gradient workspace.
+ * mmf_row_mlp_train_fwd: mmf_row_mlp (bit-identical outputs) that also writes the tape.
+ * mmf_row_mlp_bwd: the reverse program `bops` (usually the ops in reverse order) over a per-row delta scratch of
+ *   scratch_floats floats, laid out like the forward scratch.  d_outputs[i] (rows, out_dims[i]) seed slot dout_slots[i].
+ *   For each reverse op (forward op o = ops[bop.op], y = its output from the tape):
+ *       g        = delta[g : g + out_dim] * act'(y)      (ReLU: y > 0; Sigmoid: y (1 - y); none: 1)
+ *       delta[g] = g, and g -> the delta planes
+ *       delta[dres : + out_dim]  = g          or += g         (dres >= 0: the op has a residual; MMF_MLP_DRES_ACC)
+ *       delta[dsrc : + in_dim]   = W^T g      or += W^T g     (dsrc >= 0; MMF_MLP_DSRC_ACC), fp32 FFMA over j in order
+ *   then d_inputs[i] (rows, din_dims[i]) = delta[din_slots[i] ...].  weights_t holds, at each op's w_off, the torch
+ *   layout W (out_dim, in_dim) row-major followed by b (out_dim).
+ * mmf_row_mlp_weight_grads: grads at each op's w_off, torch layout like weights_t:
+ *       dW (out_dim, in_dim) = sum_rows g x^T,   db (out_dim) = sum_rows g,   x = the op's input from the tape.
+ *   The rows are split into fixed chunks whose partial sums go to `workspace` (mmf_row_mlp_train_sizes bytes); a second
+ *   kernel adds them in a fixed order: no floating-point atomics, bit-reproducible.  All outputs are overwritten. */
+/* mmf_row_mlp_weight_grads takes programs of at most MMF_MLP_MAX_DW_TILES 64 x 64 tiles, summed over the ops:
+ * ceil(out_dim / 64) * ceil(in_dim / 64). */
+#define MMF_MLP_MAX_DW_TILES 512
+#define MMF_MLP_DSRC_ACC 1
+#define MMF_MLP_DRES_ACC 2
+typedef struct mmf_mlp_bwd_op {
+  int32_t op;   /* forward op index */
+  int32_t g;    /* delta slot of the op's output: d loss / d dst on entry, g afterwards */
+  int32_t dsrc; /* delta slot of the op's input, < 0: not needed */
+  int32_t dres; /* delta slot of the op's residual, < 0: no residual */
+  int32_t flags;
+  int32_t reserved;
+} mmf_mlp_bwd_op;
+int mmf_row_mlp_train_sizes(int64_t rows, const mmf_mlp_op* ops, int32_t n_ops, int64_t* tape_floats,
+                            int64_t* delta_floats, size_t* workspace_bytes);
+int mmf_row_mlp_train_fwd(int64_t rows, const mmf_mlp_op* ops, int32_t n_ops, const float* weights,
+                          const float* const* inputs, const int32_t* in_dims, const int32_t* in_slots, int32_t n_inputs,
+                          float* const* outputs, const int32_t* out_dims, const int32_t* out_slots, int32_t n_outputs,
+                          int32_t scratch_floats, float* tape, void* stream);
+int mmf_row_mlp_bwd(int64_t rows, const mmf_mlp_op* ops, int32_t n_ops, const float* weights_t, const float* tape,
+                    const mmf_mlp_bwd_op* bops, int32_t n_bops, const float* const* d_outputs, const int32_t* out_dims,
+                    const int32_t* dout_slots, int32_t n_outputs, float* const* d_inputs, const int32_t* din_dims,
+                    const int32_t* din_slots, int32_t n_dinputs, int32_t scratch_floats, float* delta, void* stream);
+int mmf_row_mlp_weight_grads(int64_t rows, const mmf_mlp_op* ops, int32_t n_ops, const float* tape, const float* delta,
+                             float* grads, void* workspace, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -74,8 +74,15 @@ class MlpOp(C.Structure):
     ]
 
 
+class MlpBwdOp(C.Structure):
+    _fields_ = [("op", C.c_int32), ("g", C.c_int32), ("dsrc", C.c_int32), ("dres", C.c_int32), ("flags", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
 MLP_MAX_OPS, MLP_MAX_IO = 24, 4
 MLP_NONE, MLP_RELU, MLP_SIGMOID = 0, 1, 2
+MLP_DSRC_ACC, MLP_DRES_ACC = 1, 2
+MLP_MAX_DW_TILES = 512
 
 
 class MMFError(RuntimeError):
@@ -141,6 +148,19 @@ PROTOTYPES = {
         [C.c_int64, C.POINTER(MlpOp), _i32, _vp, C.POINTER(_vp), C.POINTER(_i32), C.POINTER(_i32), _i32, C.POINTER(_vp),
          C.POINTER(_i32), C.POINTER(_i32), _i32, _i32, _vp],
     ),
+    "mmf_row_mlp_train_sizes": (
+        C.c_int, [C.c_int64, C.POINTER(MlpOp), _i32, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(_sz)]),
+    "mmf_row_mlp_train_fwd": (
+        C.c_int,
+        [C.c_int64, C.POINTER(MlpOp), _i32, _vp, C.POINTER(_vp), C.POINTER(_i32), C.POINTER(_i32), _i32, C.POINTER(_vp),
+         C.POINTER(_i32), C.POINTER(_i32), _i32, _i32, _vp, _vp],
+    ),
+    "mmf_row_mlp_bwd": (
+        C.c_int,
+        [C.c_int64, C.POINTER(MlpOp), _i32, _vp, _vp, C.POINTER(MlpBwdOp), _i32, C.POINTER(_vp), C.POINTER(_i32),
+         C.POINTER(_i32), _i32, C.POINTER(_vp), C.POINTER(_i32), C.POINTER(_i32), _i32, _i32, _vp, _vp],
+    ),
+    "mmf_row_mlp_weight_grads": (C.c_int, [C.c_int64, C.POINTER(MlpOp), _i32, _vp, _vp, _vp, _vp, _vp]),
     "mmf_chain_mma_bytes": (_sz, [C.POINTER(Chain)]),
     "mmf_pack_chain_mma": (C.c_int, [C.POINTER(Chain), _vp, _vp]),
 }

@@ -3,8 +3,9 @@ constructor arguments, attributes and ``state_dict`` keys, so reference checkpoi
 reference's scripts run), wired to the CUDA kernels.
 
 The per-particle and per-trajectory arithmetic is NOT evaluated by these modules on the fused
-path: they are parameter containers whose weights ``fused.py`` packs for the kernels.  Their
-``forward`` methods are the generic (torch-on-GPU) path used when gradients are required.
+path: they are parameter containers whose weights ``fused.py`` packs for the kernels.  Under autograd
+the per-trajectory stacks train through the row-program kernels (``fused.RowProgram.run_train``); the
+rest of their ``forward`` methods is the generic (torch-on-GPU) path used when gradients are required.
 
 ref: crossmodal/base_models/*.py, crossmodal/push_models/*.py, crossmodal/door_models/*.py
 """
@@ -66,6 +67,8 @@ class _Encoders(nn.Module):
         assert len(valid | set(modalities)) == 3, "Received invalid modality"
         assert len(modalities) > 0, "Received empty modality list"
         self.modalities = set(modalities)
+        # training through the one-launch programs (fused.RowProgram.run_train); False keeps the torch modules
+        self.fused_train = True
         if "image" in self.modalities:
             self.observation_image_layers = _image_encoder(units, spanning_avg_pool)
         if "pos" in self.modalities:
@@ -113,11 +116,13 @@ class _Encoders(nn.Module):
 
         return fused.cached_program(self, key, build)
 
-    def program_inputs(self, observations):
-        """Inputs of ``encoded_program`` in its order, or None when the fused launch does not apply."""
+    def program_inputs(self, observations, prog):
+        """Inputs of ``prog`` (an ``encoded_program`` or None) in its order, or None when the fused launch does not apply:
+        decided before the image encoder runs, so that the torch path does not run it twice."""
         encs = self._encoder_list()
         raw = [observations[fused.OBS_KEY[mod]] for mod, _ in encs if mod != "image"]
-        if not fused.row_program_ok(*raw) or ("image" in self.modalities and not observations["image"].is_cuda):
+        if not (fused.row_program_ok(*raw) or fused.row_train_ok(self, *raw)) or (
+                "image" in self.modalities and not observations["image"].is_cuda) or fused.usable(prog) is None:
             return None
         return [enc(observations["image"][:, None]) if mod == "image" else observations[fused.OBS_KEY[mod]]
                 for mod, enc in encs]
@@ -211,9 +216,52 @@ class _Head(tf_base.ParticleFilterMeasurementModel, _Encoders):
         assert type(observations) == dict
         assert states.dim() == 3 and states.shape[2] == self.state_dim
         N, M, _ = states.shape
+        if M == 1:  # one state per trajectory (measurement pre-training): the whole head is a per-trajectory stack
+            out = self._train_single(states[:, 0, :], observations)
+            if out is not None:
+                return out
         f_obs = self.encode(observations)
         merged = torch.cat((f_obs[:, None, :].expand(N, M, f_obs.shape[1]), self.state_layers(states)), dim=2)
         return self.shared_layers(merged)[..., 0]
+
+
+    def _train_single(self, states, observations):
+        """(N, 1) log-likelihoods of one state per trajectory under autograd through one program -- inputs [image
+        features?, pos, sensors, states]: the encoders and ``state_layers`` write the concatenation of ``forward``, then
+        ``shared_layers`` -- or None when the training path does not apply."""
+        encs = self._encoder_list()
+        raw = [observations[fused.OBS_KEY[mod]] for mod, _ in encs if mod != "image"] + [states]
+        if not fused.row_train_ok(self, *raw) or ("image" in self.modalities and not observations["image"].is_cuda):
+            return None
+        prog = fused.usable(self.single_program())
+        if prog is None:
+            return None
+        ins = [enc(observations["image"][:, None]) if mod == "image" else observations[fused.OBS_KEY[mod]]
+               for mod, enc in encs]
+        return prog.run_train(ins + [states])[0]
+
+    def single_program(self):
+        """The program of ``_train_single`` (None: not fusable)."""
+        encs = self._encoder_list()
+
+        def build():
+            prog, u = fused.RowProgram(), self.units
+            base = prog.alloc(u * (len(encs) + 1), fresh=True)
+            for i, (mod, enc) in enumerate(encs):
+                if mod == "image":
+                    prog.input(u, slot=base + u * i)
+                else:
+                    src = prog.input(enc[0].in_features)
+                    prog.sequential(enc, src, enc[0].in_features, dst=base + u * i)
+                    prog.release(src, enc[0].in_features)
+            src = prog.input(self.state_dim)
+            prog.sequential(self.state_layers, src, self.state_dim, dst=base + u * len(encs))
+            prog.release(src, self.state_dim)
+            slot, dim = prog.sequential(self.shared_layers, base, u * (len(encs) + 1))
+            prog.output(slot, dim)
+            return prog
+
+        return fused.cached_program(self, "single", build)
 
 
 class PushMeasurementModel(_Head):  # ref: crossmodal/push_models/pf.py:30-109
@@ -276,10 +324,13 @@ class _PFWeights(CrossmodalWeightModel, _Encoders):
             nn.Linear(units, 2),
         )
 
+    def program(self):
+        return self.encoded_program("weights", [(self.fusion_layers, None, 3 * UNITS)])
+
     def forward(self, *, observations):
-        ins = self.program_inputs(observations)
-        prog = self.encoded_program("weights", [(self.fusion_layers, None, 3 * UNITS)]) if ins is not None else None
-        out = prog.run(ins)[0] if prog is not None else self.fusion_layers(self.encode(observations))
+        prog = self.program()
+        ins = self.program_inputs(observations, prog)
+        out = fused.run_program(prog, ins)[0] if ins is not None else self.fusion_layers(self.encode(observations))
         assert out.shape == (observations["gripper_pos"].shape[0], self.modality_count)
         if self.know_image_blackout:
             out[_blackout_rows(observations), 0] -= np.inf  # quirk Q3
@@ -361,13 +412,10 @@ class _VirtualSensor(tf_base.VirtualSensorModel, _Encoders):
     def forward(self, *, observations):
         # R9, ref: crossmodal/door_models/kf.py:81-126
         assert type(observations) == dict
-        ins = self.program_inputs(observations) if self.noise_R_tril is None else None
-        prog = None
-        if ins is not None:  # encoders + shared stack + both heads in one launch (mmf_row_mlp)
-            prog = self.encoded_program("sensor", [(self.shared_layers, None, self.units * len(self.modalities)),
-                                                   (self.z_layer, 0, self.units), (self.r_layer, self.units, self.units)])
-        if prog is not None:
-            z, lt_hat = prog.run(ins)
+        prog = self.program() if self.noise_R_tril is None else None  # encoders + shared stack + both heads in one launch
+        ins = self.program_inputs(observations, prog)
+        if ins is not None:
+            z, lt_hat = fused.run_program(prog, ins)
         else:
             h = self.shared_layers(self.encode(observations))
             z = self.z_layer(h[:, : self.units].clone())
@@ -376,6 +424,11 @@ class _VirtualSensor(tf_base.VirtualSensorModel, _Encoders):
         if self.add_R_noise[0] > 0:
             R = R + torch.diag(self.add_R_noise).to(R.device)
         return z, torch.sqrt(R)
+
+
+    def program(self):
+        return self.encoded_program("sensor", [(self.shared_layers, None, self.units * len(self.modalities)),
+                                               (self.z_layer, 0, self.units), (self.r_layer, self.units, self.units)])
 
 
 class PushVirtualSensorModel(_VirtualSensor):  # ref: crossmodal/push_models/kf.py:31-128
@@ -430,11 +483,14 @@ class _KFWeights(CrossmodalKalmanFilterWeightModel, _Encoders):
         )
         self.know_image_blackout = know_image_blackout
 
+    def program(self):
+        return self.encoded_program("weights", [(self.fusion_layers, None, 3 * UNITS)])
+
     def raw(self, observations):
-        ins = self.program_inputs(observations)
-        prog = self.encoded_program("weights", [(self.fusion_layers, None, 3 * UNITS)]) if ins is not None else None
-        if prog is not None:  # encoders + fusion stack + sigmoid in one launch
-            return prog.run(ins)[0]
+        prog = self.program()
+        ins = self.program_inputs(observations, prog)
+        if ins is not None:  # encoders + fusion stack + sigmoid in one launch
+            return fused.run_program(prog, ins)[0]
         return self.fusion_layers(self.encode(observations))
 
     @staticmethod

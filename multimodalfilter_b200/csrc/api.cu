@@ -480,7 +480,44 @@ int mmf_row_mlp(int64_t rows, const mmf_mlp_op* ops, int32_t n_ops, const float*
   MMF_REQUIRE(rows >= 0, "row_mlp: rows = %lld", (long long)rows);
   MMF_REQUIRE(inputs && in_dims && in_slots && outputs && out_dims && out_slots, "row_mlp: NULL argument array");
   return launch_row_mlp(rows, ops, n_ops, weights, inputs, in_dims, in_slots, n_inputs, outputs, out_dims, out_slots,
-                        n_outputs, scratch_floats, (cudaStream_t)stream);
+                        n_outputs, scratch_floats, nullptr, (cudaStream_t)stream);
+}
+
+int mmf_row_mlp_train_sizes(int64_t rows, const mmf_mlp_op* ops, int32_t n_ops, int64_t* tape_floats,
+                            int64_t* delta_floats, size_t* workspace_bytes) {
+  long long t = 0, d = 0;
+  const int rc = row_mlp_train_sizes(rows, ops, n_ops, &t, &d, workspace_bytes);
+  if (tape_floats) *tape_floats = t;
+  if (delta_floats) *delta_floats = d;
+  return rc;
+}
+
+int mmf_row_mlp_train_fwd(int64_t rows, const mmf_mlp_op* ops, int32_t n_ops, const float* weights,
+                          const float* const* inputs, const int32_t* in_dims, const int32_t* in_slots, int32_t n_inputs,
+                          float* const* outputs, const int32_t* out_dims, const int32_t* out_slots, int32_t n_outputs,
+                          int32_t scratch_floats, float* tape, void* stream) {
+  MMF_REQUIRE(rows >= 0, "row_mlp_train: rows = %lld", (long long)rows);
+  MMF_REQUIRE(inputs && in_dims && in_slots && outputs && out_dims && out_slots, "row_mlp_train: NULL argument array");
+  MMF_REQUIRE(rows == 0 || tape, "row_mlp_train: NULL tape");
+  return launch_row_mlp(rows, ops, n_ops, weights, inputs, in_dims, in_slots, n_inputs, outputs, out_dims, out_slots,
+                        n_outputs, scratch_floats, tape, (cudaStream_t)stream);
+}
+
+int mmf_row_mlp_bwd(int64_t rows, const mmf_mlp_op* ops, int32_t n_ops, const float* weights_t, const float* tape,
+                    const mmf_mlp_bwd_op* bops, int32_t n_bops, const float* const* d_outputs, const int32_t* out_dims,
+                    const int32_t* dout_slots, int32_t n_outputs, float* const* d_inputs, const int32_t* din_dims,
+                    const int32_t* din_slots, int32_t n_dinputs, int32_t scratch_floats, float* delta, void* stream) {
+  MMF_REQUIRE(rows >= 0, "row_mlp_bwd: rows = %lld", (long long)rows);
+  MMF_REQUIRE(d_outputs && out_dims && dout_slots && (n_dinputs == 0 || (d_inputs && din_dims && din_slots)),
+              "row_mlp_bwd: NULL argument array");
+  return launch_row_mlp_bwd(rows, ops, n_ops, weights_t, tape, bops, n_bops, d_outputs, out_dims, dout_slots, n_outputs,
+                            d_inputs, din_dims, din_slots, n_dinputs, scratch_floats, delta, (cudaStream_t)stream);
+}
+
+int mmf_row_mlp_weight_grads(int64_t rows, const mmf_mlp_op* ops, int32_t n_ops, const float* tape, const float* delta,
+                             float* grads, void* workspace, void* stream) {
+  MMF_REQUIRE(rows >= 0, "row_mlp_weight_grads: rows = %lld", (long long)rows);
+  return launch_row_mlp_dw(rows, ops, n_ops, tape, delta, grads, workspace, (cudaStream_t)stream);
 }
 
 size_t mmf_enc_trunk_scratch_bytes(void) { return enc_trunk_scratch_bytes(); }

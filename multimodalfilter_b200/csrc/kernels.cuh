@@ -130,7 +130,16 @@ int launch_enc_trunk(int n_images, int cout, const float* images, const void* we
                      cudaStream_t stream);
 int launch_row_mlp(long long rows, const mmf_mlp_op* ops, int n_ops, const float* weights, const float* const* inputs,
                    const int32_t* in_dims, const int32_t* in_slots, int n_inputs, float* const* outputs,
-                   const int32_t* out_dims, const int32_t* out_slots, int n_outputs, int scratch, cudaStream_t stream);
+                   const int32_t* out_dims, const int32_t* out_slots, int n_outputs, int scratch, float* tape,
+                   cudaStream_t stream);
+int row_mlp_train_sizes(long long rows, const mmf_mlp_op* ops, int n_ops, long long* tape_floats, long long* delta_floats,
+                        size_t* workspace_bytes);
+int launch_row_mlp_bwd(long long rows, const mmf_mlp_op* ops, int n_ops, const float* weights_t, const float* tape,
+                       const mmf_mlp_bwd_op* bops, int n_bops, const float* const* d_outputs, const int32_t* out_dims,
+                       const int32_t* dout_slots, int n_outputs, float* const* d_inputs, const int32_t* din_dims,
+                       const int32_t* din_slots, int n_dinputs, int scratch, float* delta, cudaStream_t stream);
+int launch_row_mlp_dw(long long rows, const mmf_mlp_op* ops, int n_ops, const float* tape, const float* delta, float* grads,
+                      void* workspace, cudaStream_t stream);
 size_t chain_mma_bytes(const mmf_chain* chain);
 int pack_chain_mma(const mmf_chain* chain, void* dst, cudaStream_t stream);
 

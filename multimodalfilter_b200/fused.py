@@ -219,14 +219,14 @@ class _HeadSpec:
     def observation_features(self, observations) -> torch.Tensor:
         """(B, feat_dim) for a dict of (B, ...) observations (ref: pf.py:76-88, order image/pos/sensors)."""
         raw = [observations[key] for key, _ in self.encoders if key != "image"]
-        if raw and row_program_ok(*raw):
-            prog = cached_program(self.head, "features", self._feature_program)
+        if raw and (row_program_ok(*raw) or row_train_ok(self.head, *raw)):
+            prog = usable(cached_program(self.head, "features", self._feature_program))
             if prog is not None:
                 ins = []
                 for key, enc in self.encoders:
                     x = observations[key]
                     ins.append(enc(x[:, None, :, :]) if key == "image" else x)
-                return prog.run(ins)[0]
+                return run_program(prog, ins)[0]
         feats = []
         for key, enc in self.encoders:
             x = observations[key]
@@ -540,10 +540,225 @@ class RowProgram:
         return ops.row_mlp(self.ops, self._weights(inputs[0].device), inputs, self.in_slots, self.out_dims, self.out_slots,
                            self.scratch)
 
+    # -- training -------------------------------------------------------------------------------------------------------
+    def parameters(self):
+        """Weight and bias of every op's Linear, in op order (the order ``training.FusedRowProgram`` takes them)."""
+        return [p for lin in self.params for p in (lin.weight, lin.bias)]
+
+    def run_train(self, inputs):
+        """``run`` under autograd: the tape-recording launch and its reverse mode (``training.FusedRowProgram``).  When
+        nothing requires a gradient it is the tape-less launch and no graph is built."""
+        from . import training
+
+        assert len(inputs) == len(self.in_slots) and all(x.shape[1] == d for x, d in zip(inputs, self.in_dims))
+        if not self.trainable():  # callers check ``usable`` first; this keeps the error out of the backward
+            raise NotFusable("the reverse program of this stack does not compile")
+        params = self.parameters()
+        if not (any(x.requires_grad for x in inputs) or any(p.requires_grad for p in params)):
+            return self.run(inputs)
+        return list(training.FusedRowProgram.apply(self, len(inputs), *inputs, *params))
+
+    def train_weights(self, device):
+        """(input-major pack of ``run``, torch-layout pack of the reverse program and the weight gradients: per op at its
+        w_off the weight (out, in) row-major, then the bias), repacked when a parameter changed."""
+        sig = (str(device), tuple((p.data_ptr(), p._version) for p in self.parameters()))
+        cached = self.__dict__.get("_packed_train")
+        if cached is None or cached[0] != sig:
+            fwd = self._weights(device)
+            bwd = torch.cat([p.detach().reshape(-1).float() for p in self.parameters()]).to(device).contiguous()
+            cached = self._packed_train = (sig, fwd, bwd)
+        return cached[1], cached[2]
+
+    def trace(self):
+        """The forward over scratch addresses: values are the program inputs (ids 0 .. n_in - 1) and the op outputs (id
+        n_in + o).  -> (values [(slot, dim)], per op (src span, res span or None), output spans), a span being the list
+        of (value, offset) of its floats."""
+        owner = [None] * self.scratch
+        values = []
+
+        def define(slot, dim):
+            v = len(values)
+            values.append((slot, dim))
+            owner[slot:slot + dim] = [(v, k) for k in range(dim)]
+
+        def span(slot, dim):
+            s = owner[slot:slot + dim]
+            if len(s) != dim or any(x is None for x in s):
+                raise NotFusable("a span reads scratch no value wrote")
+            return s
+
+        for slot, dim in zip(self.in_slots, self.in_dims):
+            define(slot, dim)
+        reads = []
+        for op in self.ops:
+            reads.append((span(op.src, op.in_dim), span(op.res, op.out_dim) if op.res >= 0 else None))
+            define(op.dst, op.out_dim)
+        outs = [span(s, d) for s, d in zip(self.out_slots, self.out_dims)]
+        return values, reads, outs
+
+    def trainable(self) -> bool:
+        """Whether the training kernels take this program: its reverse program compiles (with every input needing a
+        gradient, which a program with fewer such inputs only shrinks) and its weight gradients fit
+        ``mmf_row_mlp_weight_grads``.  Decided when the path is chosen, never inside a backward.  Cached."""
+        ok = self.__dict__.get("_trainable")
+        if ok is None:
+            tiles = sum(-(-op.out_dim // 64) * -(-op.in_dim // 64) for op in self.ops)
+            try:
+                self.reverse((True,) * len(self.in_slots))
+                ok = tiles <= _lib.MLP_MAX_DW_TILES
+            except NotFusable:
+                ok = False
+            self._trainable = ok
+        return ok
+
+    def reached(self, have_grad):
+        """(ops, inputs) that an output with a gradient depends on (``have_grad``: one flag per output).  Cached."""
+        cache = self.__dict__.setdefault("_reached_cache", {})
+        key = tuple(bool(x) for x in have_grad)
+        if key not in cache:
+            cache[key] = self._reached(key)
+        return cache[key]
+
+    def _reached(self, have_grad):
+        values, reads, outs = self.trace()
+        n_in = len(self.in_slots)
+        seen, todo = set(), [v for o, on in zip(outs, have_grad) if on for v, _ in o]
+        while todo:
+            v = todo.pop()
+            if v in seen:
+                continue
+            seen.add(v)
+            if v >= n_in:
+                src, res = reads[v - n_in]
+                todo += [u for u, _ in src] + ([u for u, _ in res] if res else [])
+        return {v - n_in for v in seen if v >= n_in}, {v for v in seen if v < n_in}
+
+    def reverse(self, need_inputs):
+        """The reverse program for ``mmf_row_mlp_bwd`` (cached per tuple of input flags): delta slots by value liveness.
+        Values read together (a concatenation read by one op, an output) form one block whose delta keeps the forward
+        layout; a block is allocated when its first consumer (in reverse) writes it and released after the last of its
+        producers has run (blocks holding an input that needs a gradient live to the end).  A consumer's write is a first
+        write when nothing wrote its range yet and an accumulation when everything did; anything else is NotFusable.
+        -> namespace(ops, dout_slots, inputs, din_slots, scratch)."""
+        cache = self.__dict__.setdefault("_reverse", {})
+        key = tuple(bool(x) for x in need_inputs)
+        if key not in cache:
+            cache[key] = self._compile_reverse(key)
+        return cache[key]
+
+    def _compile_reverse(self, need):
+        import types
+
+        values, reads, outs = self.trace()
+        n_in = len(self.in_slots)
+        parent = list(range(len(values)))
+
+        def find(v):
+            while parent[v] != v:
+                parent[v] = parent[parent[v]]
+                v = parent[v]
+            return v
+
+        for sp in [s for r in reads for s in r if s] + outs:
+            for v, _ in sp[1:]:
+                parent[find(v)] = find(sp[0][0])
+        blocks = {}
+        for v in range(len(values)):
+            blocks.setdefault(find(v), []).append(v)
+        base, size = {}, {}
+        for b, members in blocks.items():
+            spans = sorted((values[v][0], values[v][0] + values[v][1]) for v in members)
+            if any(spans[i][1] > spans[i + 1][0] for i in range(len(spans) - 1)):
+                raise NotFusable("values of one delta block overlap in the forward scratch")
+            base[b], size[b] = spans[0][0], spans[-1][1] - spans[0][0]
+        # a block dies after its earliest producer op has run, unless it holds an input that needs a gradient
+        first_producer = {b: min((v - n_in for v in m if v >= n_in), default=-1) for b, m in blocks.items()}
+        keep = {b for b, m in blocks.items() if any(v < n_in and need[v] for v in m)}
+        needed = lambda v: v >= n_in or need[v]  # noqa: E731  (values whose delta somebody uses)
+        dalloc = RowProgram()  # its slot allocator, over the delta scratch
+        slot, written = {}, {}
+
+        def place(sp, what):
+            """delta slot of a span, allocating its block; -> (slot, accumulate)."""
+            b = find(sp[0][0])
+            if b not in slot:
+                slot[b] = dalloc.alloc(size[b])
+                written[b] = [False] * size[b]
+            lo = values[sp[0][0]][0] + sp[0][1] - base[b]
+            w = written[b][lo:lo + len(sp)]
+            if any(w) and not all(w):
+                raise NotFusable(f"{what}: a delta range is partly written")
+            written[b][lo:lo + len(sp)] = [True] * len(sp)
+            return slot[b] + lo, all(w)
+
+        dout_slots = []
+        for sp in outs:
+            s, acc = place(sp, "output")
+            if acc:
+                raise NotFusable("two outputs share a value")
+            dout_slots.append(s)
+        rev = []
+        for o in reversed(range(len(self.ops))):
+            op, (src, res) = self.ops[o], reads[o]
+            v = n_in + o
+            b = find(v)
+            lo = values[v][0] - base[b]
+            if b not in slot or not all(written[b][lo:lo + op.out_dim]):
+                raise NotFusable(f"op {o}: no output with a gradient path reads its result")
+            bop = _lib.MlpBwdOp()
+            bop.op, bop.g, bop.dsrc, bop.dres, bop.flags = o, slot[b] + lo, -1, -1, 0
+            for sp, field, flag in ((res, "dres", _lib.MLP_DRES_ACC), (src, "dsrc", _lib.MLP_DSRC_ACC)):
+                if sp and any(needed(u) for u, _ in sp):
+                    if find(sp[0][0]) == b:
+                        raise NotFusable(f"op {o} reads the block it writes")
+                    s, acc = place(sp, f"op {o}")
+                    setattr(bop, field, s)
+                    bop.flags |= flag if acc else 0
+            rev.append(bop)
+            for blk, first in first_producer.items():
+                if first == o and blk not in keep:
+                    dalloc.release(slot[blk], size[blk])
+        # inputs whose delta nobody wrote (no op or output reads them) are left out: they receive no gradient
+        inputs, din_slots = [], []
+        for i in range(n_in):
+            b = find(i)
+            lo = values[i][0] - base.get(b, 0)
+            if need[i] and b in slot and all(written[b][lo:lo + values[i][1]]):
+                inputs.append(i)
+                din_slots.append(slot[b] + lo)
+        if dalloc.scratch > 1536:
+            raise NotFusable("delta scratch too large")
+        return types.SimpleNamespace(ops=rev, dout_slots=dout_slots, inputs=inputs, din_slots=din_slots,
+                                     scratch=max(dalloc.scratch, 4))
+
 
 def row_program_ok(*tensors) -> bool:
     """The one-launch programs serve inference on CUDA fp32 rows; anything else keeps the torch modules."""
     return not torch.is_grad_enabled() and all(t.is_cuda and t.dtype == torch.float32 and t.dim() == 2 for t in tensors)
+
+
+def row_train_ok(owner, *tensors) -> bool:
+    """The programs under autograd (``RowProgram.run_train``): grad mode on, CUDA fp32 2-D rows, ``owner.fused_train``
+    (default on) and no forward or pre-forward hook on ``owner`` or its submodules (the fused launch never calls those
+    modules).  Anything else keeps the torch modules."""
+    if not torch.is_grad_enabled() or not getattr(owner, "fused_train", True):
+        return False
+    if not all(isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float32 and t.dim() == 2 for t in tensors):
+        return False
+    return not any(m._forward_hooks or m._forward_pre_hooks for m in owner.modules())
+
+
+def usable(prog):
+    """``prog`` if the launch that runs now can take it (under grad mode: ``prog.trainable()``), else None: the caller
+    keeps the torch modules."""
+    if prog is None or (torch.is_grad_enabled() and not prog.trainable()):
+        return None
+    return prog
+
+
+def run_program(prog, inputs):
+    """``prog`` over ``inputs``: the training launch under grad mode, the inference launch otherwise."""
+    return prog.run_train(inputs) if torch.is_grad_enabled() else prog.run(inputs)
 
 
 def cached_program(owner, key, build):

@@ -244,6 +244,70 @@ def row_mlp(program_ops, weights, inputs, in_slots, out_dims, out_slots, scratch
     return outs
 
 
+def row_mlp_train_sizes(program_ops, rows):
+    """-> (tape floats, delta-plane floats, weight-gradient workspace bytes) of a program over ``rows`` rows."""
+    lib = _lib.load()
+    t, d, w = C.c_int64(), C.c_int64(), C.c_size_t()
+    op_arr = (_lib.MlpOp * len(program_ops))(*program_ops)
+    _lib.check(lib.mmf_row_mlp_train_sizes(rows, op_arr, len(program_ops), C.byref(t), C.byref(d), C.byref(w)))
+    return t.value, d.value, w.value
+
+
+def row_mlp_train_fwd(program_ops, weights, inputs, in_slots, out_dims, out_slots, scratch):
+    """``row_mlp`` that also records the tape of ``row_mlp_bwd`` (layout: include/mmf_b200.h) -> (outputs, tape)."""
+    lib = _lib.load()
+    rows = inputs[0].shape[0]
+    inputs = [_f32c(x) for x in inputs]
+    assert all(x.dim() == 2 and x.shape[0] == rows for x in inputs)
+    dev = inputs[0].device
+    outs = [torch.empty((rows, d), device=dev, dtype=torch.float32) for d in out_dims]
+    tape = torch.empty(row_mlp_train_sizes(program_ops, rows)[0], device=dev, dtype=torch.float32)
+    n_ops, n_in, n_out = len(program_ops), len(inputs), len(outs)
+    op_arr = (_lib.MlpOp * n_ops)(*program_ops)
+    in_ptrs = (C.c_void_p * n_in)(*[x.data_ptr() for x in inputs])
+    in_dims = (C.c_int32 * n_in)(*[x.shape[1] for x in inputs])
+    out_ptrs = (C.c_void_p * n_out)(*[o.data_ptr() for o in outs])
+    for x in inputs:
+        _lib.ptr(x)
+    _lib.check(PROFILE.run("row_mlp_train", 1, lib.mmf_row_mlp_train_fwd, rows, op_arr, n_ops, _lib.ptr(weights), in_ptrs,
+                           in_dims, (C.c_int32 * n_in)(*in_slots), n_in, out_ptrs, (C.c_int32 * n_out)(*out_dims),
+                           (C.c_int32 * n_out)(*out_slots), n_out, scratch, _lib.ptr(tape), _lib.stream_of(inputs[0])))
+    return outs, tape
+
+
+def row_mlp_bwd(program_ops, weights_t, tape, rev_ops, d_outputs, dout_slots, din_dims, din_slots, scratch):
+    """Reverse program of ``row_mlp_train_fwd``: d_outputs (rows, d_i) -> (d_inputs (rows, din_dims[i]), delta planes)."""
+    lib = _lib.load()
+    rows = d_outputs[0].shape[0]
+    d_outputs = [_f32c(x) for x in d_outputs]
+    dev = tape.device
+    d_in = [torch.empty((rows, d), device=dev, dtype=torch.float32) for d in din_dims]
+    delta = torch.empty(row_mlp_train_sizes(program_ops, rows)[1], device=dev, dtype=torch.float32)
+    n_ops, n_b, n_out, n_din = len(program_ops), len(rev_ops), len(d_outputs), len(d_in)
+    for x in d_outputs:
+        _lib.ptr(x)
+    _lib.check(PROFILE.run(
+        "row_mlp_bwd", 1, lib.mmf_row_mlp_bwd, rows, (_lib.MlpOp * n_ops)(*program_ops), n_ops, _lib.ptr(weights_t),
+        _lib.ptr(tape), (_lib.MlpBwdOp * n_b)(*rev_ops), n_b, (C.c_void_p * n_out)(*[x.data_ptr() for x in d_outputs]),
+        (C.c_int32 * n_out)(*[x.shape[1] for x in d_outputs]), (C.c_int32 * n_out)(*dout_slots), n_out,
+        (C.c_void_p * max(n_din, 1))(*[x.data_ptr() for x in d_in]), (C.c_int32 * max(n_din, 1))(*din_dims),
+        (C.c_int32 * max(n_din, 1))(*din_slots), n_din, scratch, _lib.ptr(delta), _lib.stream_of(tape)))
+    return d_in, delta
+
+
+def row_mlp_weight_grads(program_ops, rows, tape, delta, pack_floats):
+    """dW, db of every op of a program from the tape and the delta planes, as one flat pack in the torch layout of the
+    weights (per op at its w_off: weight (out, in) row-major, then bias).  Deterministic (fixed-order reduction)."""
+    lib = _lib.load()
+    dev = tape.device
+    grads = torch.empty(pack_floats, device=dev, dtype=torch.float32)
+    ws = torch.empty(max(row_mlp_train_sizes(program_ops, rows)[2], 16), dtype=torch.uint8, device=dev)
+    n_ops = len(program_ops)
+    _lib.check(PROFILE.run("row_mlp_dw", 2, lib.mmf_row_mlp_weight_grads, rows, (_lib.MlpOp * n_ops)(*program_ops), n_ops,
+                           _lib.ptr(tape), _lib.ptr(delta), _lib.ptr(grads), _lib.ptr(ws), _lib.stream_of(tape)))
+    return grads
+
+
 def pf_init(mean, covariance, eps_MNsd):
     """R2: (N,sd), (N,sd,sd), (M,N,sd) -> particle_states (N,M,sd), particle_log_weights (N,M)."""
     lib = _lib.load()

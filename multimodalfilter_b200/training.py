@@ -288,6 +288,55 @@ class FusedDynamicsRollout(torch.autograd.Function):
         return (None, d_x0 if ctx.needs_input_grad[1] else None, d_rows if ctx.needs_input_grad[2] else None, *grads)
 
 
+class FusedRowProgram(torch.autograd.Function):
+    """(prog, n_in, inputs..., the weight and bias of every op's Linear in ``prog.parameters()`` order) -> the program's
+    outputs: a per-trajectory MLP stack (``fused.RowProgram``) in one launch that records the tape
+    (``mmf_row_mlp_train_fwd``), its reverse program in one more (``mmf_row_mlp_bwd``) and the weight gradients in two
+    (``mmf_row_mlp_weight_grads``).  Outputs without a gradient are seeded with zeros; inputs and parameters that no
+    output with a gradient reaches get None, as under autograd through the modules.  The outputs are not saved (callers
+    may edit them in place); the torch-layout weights of this forward are, so a later optimiser step does not leak into
+    the backward."""
+
+    @staticmethod
+    def forward(ctx, prog, n_in, *tensors):
+        inputs = [x.detach() for x in tensors[:n_in]]
+        w_fwd, w_t = prog.train_weights(inputs[0].device)
+        outs, tape = ops.row_mlp_train_fwd(prog.ops, w_fwd, inputs, prog.in_slots, prog.out_dims, prog.out_slots,
+                                           prog.scratch)
+        ctx.prog, ctx.n_in, ctx.w_t, ctx.tape, ctx.rows = prog, n_in, w_t, tape, inputs[0].shape[0]
+        ctx.set_materialize_grads(False)
+        return tuple(outs)
+
+    @staticmethod
+    def backward(ctx, *d_outs):
+        prog, n_in = ctx.prog, ctx.n_in
+        n_par = len(prog.ops) * 2
+        have = [d is not None for d in d_outs]
+        if not any(have):
+            return (None,) * (2 + n_in + n_par)
+        ops_reached, inputs_reached = prog.reached(have)
+        rev = prog.reverse(ctx.needs_input_grad[2:2 + n_in])
+        d = [x.contiguous() if x is not None else ctx.tape.new_zeros((ctx.rows, dim)) for x, dim in zip(d_outs, prog.out_dims)]
+        d_in, delta = ops.row_mlp_bwd(prog.ops, ctx.w_t, ctx.tape, rev.ops, d, rev.dout_slots,
+                                      [prog.in_dims[i] for i in rev.inputs], rev.din_slots, rev.scratch)
+        grads_in = [None] * n_in
+        for i, g in zip(rev.inputs, d_in):
+            grads_in[i] = g if i in inputs_reached else None
+        need = ctx.needs_input_grad[2 + n_in:]
+        grads_p = [None] * n_par
+        if any(need):
+            pack = ops.row_mlp_weight_grads(prog.ops, ctx.rows, ctx.tape, delta, prog._w_floats)
+            for o, op in enumerate(prog.ops):
+                if o not in ops_reached:
+                    continue
+                nw = op.out_dim * op.in_dim
+                if need[2 * o]:
+                    grads_p[2 * o] = pack[op.w_off:op.w_off + nw].view(op.out_dim, op.in_dim)
+                if need[2 * o + 1]:
+                    grads_p[2 * o + 1] = pack[op.w_off + nw:op.w_off + nw + op.out_dim]
+        return (None, None, *grads_in, *grads_p)
+
+
 def _dynamics_plan(dyn):
     """The packed-weight plan of a dynamics model (shared with ``DynamicsModel.jacobian``), or False if unrecognised."""
     plan = dyn.__dict__.get("_mmf_jac_plan")
